@@ -1,7 +1,7 @@
 #!/usr/bin/env python
 """bench.py — BASELINE.json metric: text-line-crops/sec (recognition), config 2.
 
-    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference]
+    python bench.py [--gpus N] [--steps K] [--warmup W] [--impl reference] [--dump-outputs DIR]
 
 Workload (BASELINE config 2 / SURVEY.md §8d): B = 256 synthetic 48x512 uint8 line crops per GPU -> 56x560,
 160 patches, 46-token prompt each; declared synthetic model SYN-REC (vision tower = reference defaults,
@@ -23,8 +23,10 @@ sb_rec_preprocess on the device vs the OpenCV thread pool; N = 1 only), `ocr_err
 
 Multi-GPU (torchrun, one rank per GPU): replicas over independent crop batches (weak scaling); one NCCL
 broadcast of the packed weights at init, one all_gather of the result tensors per step.
-`--impl reference` times the reference algorithm's CPU path (the oracle port: /root/reference is not on the GPU
-box and the reference is Python, so there is nothing to compile) on all host threads, same metric/config.
+`--impl reference` times the reference algorithm's CPU path (the oracle port: the reference is Python, so there is nothing
+to compile) on all host threads, same metric/config.
+`--dump-outputs DIR` writes what the timed path returned in its last step (rank 0's replica) as DIR/{tokens,scores,bboxes}.npy;
+the inputs and weights are seeded, so two builds run with the same arguments can be compared output for output.
 """
 from __future__ import annotations
 
@@ -251,6 +253,19 @@ def gpu_eager_baseline(dev, steps_rec=MAX_TOKENS):
     out["detection"] = {"value": 32 / (ms * 1e-3), "unit": "pages/s", "ms_per_step": ms, "dtype": "f16",
                         "what": "oracle/det_oracle.py on cuda: cuDNN convolutions (NCHW, eager), BatchNorm not folded"}
     return out
+
+
+def dump_outputs(out_dir, prefill: dict, hist: dict) -> None:
+    """Tokens / scores / boxes of one resident step laid out as RecognitionRunner.run_preprocessed returns them ([crops, MAX_TOKENS]
+    and [crops, MAX_TOKENS, 6], the prefill's token first): integers as float64 (exact), scores as float32.  1.9 MB at B = 256."""
+    d = Path(out_dir)
+    d.mkdir(parents=True, exist_ok=True)
+    arrays = {"tokens": torch.cat([prefill["tok"][None], hist["tok"]], 0).T.double(),
+              "scores": torch.cat([prefill["score"][None], hist["score"]], 0).T.float(),
+              "bboxes": torch.cat([prefill["bbox"][None], hist["bbox"]], 0).transpose(0, 1).double()}
+    for name, t in arrays.items():
+        np.save(d / f"{name}.npy", t.contiguous().cpu().numpy())
+    log(f"outputs of the last timed step written to {d}")
 
 
 def _config(n_gpus):
@@ -593,7 +608,12 @@ def main():
     ap.add_argument("--no-layout", action="store_true", help="skip the layout / table_rec (config 4) secondary numbers")
     ap.add_argument("--no-pipeline", action="store_true", help="skip the ocr_text pipeline (config 5) secondary number")
     ap.add_argument("--no-ocr-error", action="store_true", help="skip the ocr_error (DistilBERT) secondary number")
+    ap.add_argument("--dump-outputs", metavar="DIR", help="write the last timed step's tokens / scores / boxes as DIR/<name>.npy")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "b200":
+        ap.error("--dump-outputs needs --impl b200")
     if args.impl == "reference":
         return run_reference_arm(args)
     args.warmup = max(args.warmup, 3)
@@ -661,8 +681,11 @@ def main():
             "done": torch.empty((MAX_TOKENS - 1, B_PER_GPU), dtype=torch.uint8, device=dev)}
     from surya_b200 import shard
 
+    last = {}
+
     def resident_step():
         out = eng.prefill(tiles_dev, plan)
+        last["prefill"] = out
         ids_io.copy_(out["next_ids"])
         pos_io.copy_(lens)
         eng.decode_steps(ids_io, slot_t, pos_io, MAX_TOKENS - 1, hist=hist, max_pos=max_len)
@@ -702,6 +725,8 @@ def main():
     ms_total = timed(resident_step, args.steps)
     launches = _lib.launch_count() - l0
     ms_step = ms_total / args.steps
+    if args.dump_outputs and rank == 0:
+        dump_outputs(args.dump_outputs, last["prefill"], hist)
     value = B_PER_GPU * world * args.steps / (ms_total * 1e-3)
 
     # ---- phase split (CUDA events, rank-local, outside the headline region)

@@ -1,8 +1,8 @@
 """ORACLE TOOLING — generate golden vectors from the reference's own nn.Modules (run in the build container).
 
-    python -m oracle.make_golden            # writes tests/golden/rec_*.pt
+    SURYA_REFERENCE=<reference checkout> python -m oracle.make_golden [rec det layout table trace ocr_error host]
 
-The reference (imported unmodified from /root/reference through oracle/ref_shim.py) is instantiated for a
+The reference (imported unmodified from the SURYA_REFERENCE checkout through oracle/ref_shim.py) is instantiated for a
 declared config, loaded with surya_b200.synth's seeded weights, and driven exactly like
 RecognitionPredictor.prefill/decode drive it (surya/recognition/__init__.py:326-352, 398-409): one prefill
 with a fresh cache, then greedy decode steps feeding process_outputs' input_ids back.  Outputs are stored in
@@ -190,8 +190,10 @@ def make_layout_variants_golden():
             cur = tok.unsqueeze(1)
             toks.append(tok)
             heads.append({k: v[:, -1].float().clone() for k, v in logits.items()})
-    g = {"encoder": ref_enc.float().clone(), "prompt": ids, "tokens": torch.stack(toks, 1),
-         "heads": {k: torch.stack([h[k] for h in heads], 1) for k in heads[0]},
+    # a seeded sample of the 2 x 128 encoder rows keeps the fixture small; the decoder heads depend on all of them
+    rows = torch.from_numpy(np.sort(np.random.default_rng(0).choice(2 * 128, size=16, replace=False)))
+    g = {"encoder_rows": rows, "encoder": ref_enc.float().reshape(2 * 128, -1)[rows].clone(), "encoder_shape": tuple(ref_enc.shape),
+         "prompt": ids, "tokens": torch.stack(toks, 1), "heads": {k: torch.stack([h[k] for h in heads], 1) for k in heads[0]},
          "meta": {"kind": "table_nonsquare_cellpass", "steps": steps, "seed": 3, "page_seed": 21, "image_size": [256, 512],
                   "torch": str(torch.__version__), "reference": "VikParuchuri/surya@80e9a7e (v0.14.6), fp32 CPU"}}
     torch.save(g, GOLDEN / "table_nonsquare_cellpass.pt")
@@ -248,6 +250,164 @@ def make_predictor_trace_golden():
           f"tokens[0]={tokens[0]}")
 
 
+def preproc_crops():
+    """Seeded uint8 crops for the crop-chain pin against the reference's SuryaOCRProcessor."""
+    rng = np.random.default_rng(11)
+    return [rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
+            for h, w in ((48, 512), (40, 300), (300, 2000), (20, 60), (56, 560), (97, 1403))]
+
+
+def det_postprocess_maps():
+    """Synthetic 512x640 heat maps of text-line-shaped blobs, 16-bit valued like the engine's maps (3 trials)."""
+    import cv2
+
+    rng = np.random.default_rng(5)
+    maps = []
+    for _ in range(3):
+        m = np.zeros((512, 640), np.float32)
+        for _ in range(25):
+            x, y = int(rng.integers(0, 560)), int(rng.integers(0, 480))
+            w, h = int(rng.integers(30, 200)), int(rng.integers(6, 24))
+            m[y:y + h, x:x + w] = rng.uniform(0.3, 1.0)
+        maps.append(cv2.GaussianBlur(m, (0, 0), 2.0).astype(np.float16).astype(np.float32))
+    return maps
+
+
+def pipeline_host_cases():
+    """(heat map, image size, page or None) for the page-polygon / polygon-slice pin: trial 1 is rescaled to twice the map size
+    and has no page; the others slice a random float32 page."""
+    import cv2
+
+    rng = np.random.default_rng(9)
+    H, W = 512, 640
+    cases = []
+    for trial in range(3):
+        m = np.zeros((H, W), np.float32)
+        for _ in range(20):
+            x, y = int(rng.integers(0, W - 60)), int(rng.integers(0, H - 30))
+            w, h = int(rng.integers(30, 220)), int(rng.integers(6, 30))
+            m[y:y + h, x:x + w] = rng.uniform(0.3, 1.0)
+        m[40:60, 100:300] = 0.9
+        m[44:56, 150:250] = 0.95                                   # a box contained in another one
+        m = cv2.GaussianBlur(m, (0, 0), 1.5).astype(np.float16).astype(np.float32)
+        img_size = (W * 2, H * 2) if trial == 1 else (W, H)
+        page = rng.integers(0, 256, size=(H, W, 3)).astype(np.float32) if trial != 1 else None
+        cases.append((m, img_size, page))
+    return cases
+
+
+def ocr_error_texts():
+    """Seeded word strings for the OCRErrorPredictor pin (8 texts of 2..29 words)."""
+    rng = np.random.default_rng(0)
+    words = [f"w{i}" for i in range(300)]
+    return [" ".join(rng.choice(words, size=int(rng.integers(2, 30)))) for _ in range(8)]
+
+
+def array_digest(a) -> str:
+    """sha256 of an array's dtype, shape and bytes: exact equality of large outputs without storing them."""
+    import hashlib
+
+    a = np.ascontiguousarray(a)
+    return hashlib.sha256(f"{a.dtype}{a.shape}".encode() + a.tobytes()).hexdigest()
+
+
+def make_reference_host_golden():
+    """What the reference's own host code and predictor classes return on seeded inputs, so that the oracle restatements and the
+    product's host stages stay pinned to the reference without the reference installed:
+      crop_chain   SuryaOCRProcessor.scale_to_fit + _process_and_tile (grids, per-row sums and sums of squares, a seeded sample
+                   of tile rows)
+      det_boxes    surya.detection.heatmap get_dynamic_thresholds / detect_boxes
+      page_polys   get_and_clean_boxes + the predictor's box expansion, and slice_polys_from_image (digests of the slices)
+      det_config1  DetectionPredictor over the reference EfficientViT on the reference's own 1024x1024 test page (BASELINE
+                   config 1): polygons, confidences and a seeded sample of the segmentation logits
+      ocr_error    OCRErrorPredictor over the reference DistilBERT: labels of 8 texts, batches of 3
+      rec_rerun    tokens of a second, shorter RecognitionPredictor run over the predictor-trace crops (see
+                   make_predictor_trace_golden)
+    """
+    from oracle import ocr_error_oracle as E
+    from oracle import ref_predictors as RP
+    from surya_b200 import dropin
+    from surya_b200.config import det_default, ocr_error_tiny
+    from surya_b200.synth import det_normalize, det_state_dict, ocr_error_state_dict
+
+    RP.install_predictors()
+    from surya.detection import DetectionPredictor
+    from surya.detection.heatmap import detect_boxes, get_and_clean_boxes, get_dynamic_thresholds
+    from surya.input.processing import slice_polys_from_image
+    from surya.settings import settings
+
+    g = {"meta": {"kind": "reference_host", "torch": str(torch.__version__),
+                  "reference": "VikParuchuri/surya@80e9a7e (v0.14.6), CPU"}}
+    cfg = tiny_rec()
+    proc = RP.synthetic_ocr_processor(cfg)
+    sample = np.random.default_rng(0)
+    g["crop_chain"] = []
+    for crop in preproc_crops():
+        tiles, grid = proc._process_and_tile(proc.scale_to_fit(np.asarray(crop, dtype=np.float32), (1024, 256)))
+        tiles = tiles.numpy()
+        rows = np.sort(sample.choice(tiles.shape[0], size=min(4, tiles.shape[0]), replace=False))
+        g["crop_chain"].append({"shape": tuple(crop.shape), "grid": tuple(int(v) for v in grid), "rows": torch.from_numpy(rows),
+                                "tile_rows": torch.from_numpy(tiles[rows].copy()),
+                                "row_sums": torch.from_numpy(tiles.astype(np.float64).sum(1)),
+                                "row_sq": torch.from_numpy((tiles.astype(np.float64) ** 2).sum(1))})
+
+    g["det_boxes"] = []
+    for m in det_postprocess_maps():
+        tt, low = get_dynamic_thresholds(m, 0.6, 0.35)
+        boxes, conf = detect_boxes(m, 0.6, 0.35)
+        g["det_boxes"].append({"map_digest": array_digest(m), "thresholds": (float(tt), float(low)),
+                               "boxes": [torch.from_numpy(np.array(b)) for b in boxes],
+                               "conf": torch.from_numpy(np.asarray(conf, dtype=np.float64))})
+
+    g["page_polys"] = []
+    for m, img_size, page in pipeline_host_cases():
+        H, W = m.shape
+        ref = get_and_clean_boxes(m, [W, H], img_size)
+        for box in ref:
+            if box.height < 3 * box.width:
+                box.expand(x_margin=0, y_margin=settings.DETECTOR_BOX_Y_EXPAND_MARGIN)
+                box.fit_to_bounds([0, 0, img_size[0], img_size[1]])
+        polys = [[[float(v) for v in pt] for pt in r.polygon] for r in ref]
+        slices = None
+        if page is not None:
+            slices = [array_digest(s) for s in slice_polys_from_image(page, [[[int(v) for v in pt] for pt in p] for p in polys])]
+        g["page_polys"].append({"map_digest": array_digest(m), "polygons": polys, "conf": [float(r.confidence) for r in ref],
+                                "slice_digests": slices})
+
+    dcfg = det_default()
+    dsd = det_state_dict(dcfg, seed=0)
+    dmodel = ref_shim.build_reference_det_model(dcfg, dsd)
+    dproc = RP.synthetic_det_processor(1024)
+    page = RP.conftest_page(1024)
+    stock = type("StockDetectionPredictor", (DetectionPredictor,), {"model_loader_cls": dropin.loader_for(dmodel, dproc)})(
+        device="cpu", dtype=torch.float32)
+    stock.disable_tqdm = True
+    res = stock([page])[0]
+    x = torch.from_numpy(dproc(np.asarray(page, dtype=np.uint8))["pixel_values"][0])[None]
+    assert (x - det_normalize(np.asarray(page, dtype=np.uint8)[None])).abs().max().item() < 1e-6
+    with torch.inference_mode():
+        logits = dmodel(pixel_values=x).logits.float()[0]
+    idx = torch.from_numpy(np.sort(sample.choice(logits[0].numel(), size=4096, replace=False)).astype(np.int32))
+    g["det_config1"] = {"page_digest": array_digest(np.asarray(page, dtype=np.uint8)), "image_bbox": list(res.image_bbox),
+                        "polygons": [[[float(v) for v in pt] for pt in b.polygon] for b in res.bboxes],
+                        "conf": [float(b.confidence) for b in res.bboxes], "logit_index": idx,
+                        "logits": logits.reshape(logits.shape[0], -1)[:, idx].clone(), "logits_shape": tuple(logits.shape)}
+
+    ecfg = ocr_error_tiny()
+    emodel = ref_shim.build_reference_ocr_error_model(ecfg, ocr_error_state_dict(ecfg, seed=0))
+    from surya.ocr_error import OCRErrorPredictor      # after install() has re-applied the tokenizer-helper names
+
+    texts = ocr_error_texts()
+    stock = type("StockOCRErrorPredictor", (OCRErrorPredictor,), {"model_loader_cls": dropin.loader_for(emodel, E.HashTokenizer(ecfg))})(
+        device="cpu", dtype=torch.float32)
+    stock.disable_tqdm = True
+    g["ocr_error"] = {"texts": texts, "batch_size": 3, "labels": list(stock(texts, batch_size=3).labels)}
+    _, rerun, *_ = RP.record_rec_trace(cfg, rec_state_dict(cfg, seed=0), trace_crops()[:4], batch_size=3, max_tokens=4)
+    g["rec_rerun"] = {"n_crops": 4, "batch_size": 3, "max_tokens": 4, "tokens": rerun}
+    torch.save(g, GOLDEN / "reference_host.pt")
+    print(f"[golden] reference_host: {len(g['det_config1']['polygons'])} config-1 polygons, ocr_error labels {g['ocr_error']['labels']}")
+
+
 def make_swin_window_padding_golden():
     """Oracle pin for DonutSwinLayer.maybe_pad (donut/encoder.py:591-596, crop :657-659): a 288x352 input gives token grids
     72x88 / 36x44 / 18x22 / 9x11 -- every merge sees even sides (the reference's floor-sized stage position tables demand it) but
@@ -293,7 +453,7 @@ def make_ocr_error_golden():
 def main():
     GOLDEN.mkdir(parents=True, exist_ok=True)
     torch.set_num_threads(8)
-    which = set(sys.argv[1:]) or {"rec", "det", "layout", "table", "trace", "ocr_error"}
+    which = set(sys.argv[1:]) or {"rec", "det", "layout", "table", "trace", "ocr_error", "host"}
     if "layout" in which:
         make_layout_golden()
     if "table" in which:
@@ -306,6 +466,8 @@ def main():
         make_predictor_trace_golden()
     if "ocr_error" in which:
         make_ocr_error_golden()
+    if "host" in which:
+        make_reference_host_golden()
     if "rec" not in which:
         return
     for kind, cfg, steps in (("tiny", tiny_rec(), 32), ("synrec", syn_rec(), 40)):

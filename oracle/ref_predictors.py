@@ -10,7 +10,7 @@
                               B200SuryaModel + SlotCache (the drop-in boundary code) in a container without a GPU
   * record_rec_trace          run RecognitionPredictor.prediction_loop and log every model call / cache operation, so the
                               GPU tests can replay the exact call sequence against the CUDA engine (tests/golden/
-                              rec_predictor_trace.pt; /root/reference does not exist on the GPU box)
+                              rec_predictor_trace.pt; the tests run without the reference)
 
 Only tests/ and oracle/make_golden.py import this module.
 """

@@ -1,25 +1,29 @@
-"""ORACLE TOOLING (build container only) — import the *unmodified* reference from /root/reference.
+"""ORACLE TOOLING (golden regeneration only) — import the *unmodified* reference surya from a checkout named by SURYA_REFERENCE.
 
 The reference pins transformers ^4.51 (pyproject.toml:15); this image has 5.5.  The few names that moved are
 patched *in transformers' namespace before import* (SURVEY.md §8c); no reference source is copied or edited.
-/root/reference does not exist on the GPU box: only oracle/make_golden.py (run here) uses this module.
+The tests never import the reference: what they compare against is stored under tests/golden/ by oracle/make_golden.py.
 """
 from __future__ import annotations
 
+import os
 import sys
 import types
 from pathlib import Path
 
-REFERENCE = Path("/root/reference")
+REFERENCE = Path(os.environ.get("SURYA_REFERENCE", "")).expanduser()
 
 
 def available() -> bool:
-    return (REFERENCE / "surya" / "__init__.py").exists()
+    try:
+        return bool(os.environ.get("SURYA_REFERENCE")) and (REFERENCE / "surya" / "__init__.py").is_file()
+    except OSError:
+        return False
 
 
 def install() -> None:
     if not available():
-        raise RuntimeError("/root/reference is not mounted: goldens can only be regenerated in the build container")
+        raise RuntimeError("set SURYA_REFERENCE to a checkout of the reference surya (VikParuchuri/surya@80e9a7e) to regenerate goldens")
     if str(REFERENCE) not in sys.path:
         sys.path.insert(0, str(REFERENCE))
     import torch

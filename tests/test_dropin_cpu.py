@@ -1,12 +1,10 @@
 """Drop-in boundary (SURVEY.md §8b) on CPU.
 
-Two kinds of tests:
-  * with /root/reference mounted (build container): the reference's UNMODIFIED predictor classes run on top of the B200 model
-    mirrors (B200SuryaModel + SlotCache, B200EfficientViT) bound through surya_b200.dropin; the engine behind the mirror is the
-    CPU oracle (oracle/ref_predictors.py) because this container has no GPU.  These are the `test_reference_*predictor_dropin*`
-    tests; they skip on the GPU box, where /root/reference does not exist.
-  * everywhere: the committed trace of such a predictor run (tests/golden/rec_predictor_trace.pt) is replayed against the same
-    boundary code without the reference.  tests/test_rec_gpu.py replays the same trace against the CUDA engine.
+The reference's UNMODIFIED predictor classes were run over the B200 model mirrors (B200SuryaModel + SlotCache, B200EfficientViT)
+with the CPU oracle as the engine, and its host post-processing on seeded heat maps; oracle/make_golden.py stored what they
+returned under tests/golden/ (rec_predictor_trace.pt, reference_host.pt).  These tests hold the oracle, the boundary code and the
+product's host stages to those outputs without the reference installed.  tests/test_rec_gpu.py replays the same predictor trace
+against the CUDA engine.
 """
 from pathlib import Path
 
@@ -15,11 +13,9 @@ import pytest
 import torch
 
 from oracle import rec_oracle as O
-from oracle import ref_shim
 
 ROOT = Path(__file__).resolve().parent.parent
 GOLDEN = ROOT / "tests" / "golden"
-needs_reference = pytest.mark.skipif(not ref_shim.available(), reason="/root/reference is only mounted in the build container")
 
 
 def _tile_fn(cfg):
@@ -29,13 +25,11 @@ def _tile_fn(cfg):
     return fn
 
 
-@needs_reference
 def test_reference_recognition_predictor_dropin_cpu():
-    """RecognitionPredictor.prediction_loop (reference code, unmodified: prefill with its own `ContinuousBatchingCache()`,
-    merge, mask/position bookkeeping, maybe_trim_cache_padding, stop rules, `del self.kv_cache`) over B200SuryaModel +
-    SlotCache: every crop must decode exactly as the oracle decodes it alone, merges must see both offset signs, and all KV
-    slots must be back in the engine afterwards."""
-    from oracle import ref_predictors as RP
+    """What RecognitionPredictor.prediction_loop (reference code, unmodified: prefill with its own `ContinuousBatchingCache()`,
+    merge, mask/position bookkeeping, maybe_trim_cache_padding, stop rules, `del self.kv_cache`) returned over B200SuryaModel +
+    SlotCache (tests/golden/rec_predictor_trace.pt, reference_host.pt): every crop decodes exactly as the oracle decodes it alone, the run merged
+    with both offset signs and trimmed, and a second, shorter run gave the same token prefixes."""
     from oracle.make_golden import trace_crops
     from surya_b200.config import tiny_rec
     from surya_b200.synth import rec_state_dict
@@ -43,23 +37,19 @@ def test_reference_recognition_predictor_dropin_cpu():
     cfg = tiny_rec()
     sd = rec_state_dict(cfg, seed=0)
     crops = trace_crops()
-    events, tokens, bboxes, scores, eng = RP.record_rec_trace(cfg, sd, crops, batch_size=3, max_tokens=10, min_trim_length=2)
+    g = torch.load(GOLDEN / "rec_predictor_trace.pt")
+    events, tokens, bboxes, scores = g["events"], g["tokens"], g["bboxes"], g["scores"]
     offsets = [e["offset"] for e in events if e["kind"] == "merge"]
     assert any(o > 0 for o in offsets) and any(o < 0 for o in offsets), offsets
     assert any(e["kind"] == "trim" for e in events)
-    assert len(eng.free_slots) == eng.max_slots, "KV slots leaked by the predictor run"
+    assert len(tokens) == len(crops)
     for i, crop in enumerate(crops):
         otok, osc, obox, hist = O.greedy_decode(sd, cfg, O.build_batch([crop], cfg), 10, torch.float32, stop_rules=True)
         assert tokens[i] == hist[0], f"crop {i}: {tokens[i]} vs oracle {hist[0]}"
         assert np.allclose(scores[i], osc[0, : len(hist[0])].numpy(), atol=1e-5)
-        assert torch.equal(bboxes[i, : len(hist[0])].long(), obox[0, : len(hist[0])])
-    # the committed fixture is what this run produces
-    g = torch.load(GOLDEN / "rec_predictor_trace.pt")
-    assert g["tokens"] == tokens
-    assert [e["kind"] for e in g["events"]] == [e["kind"] for e in events]
-    # a second loop on the same engine must find every slot free again (ADVICE r1: slot leak through `del self.kv_cache`)
-    events2, tokens2, *_ = RP.record_rec_trace(cfg, sd, crops[:4], batch_size=3, max_tokens=4)
-    assert tokens2 == [t[:4] for t in tokens[:4]]
+        assert torch.equal(torch.as_tensor(bboxes[i][: len(hist[0])]).long(), obox[0, : len(hist[0])])
+    rerun = torch.load(GOLDEN / "reference_host.pt")["rec_rerun"]
+    assert rerun["tokens"] == [t[: rerun["max_tokens"]] for t in tokens[: rerun["n_crops"]]]
 
 
 def test_predictor_trace_replay_cpu():
@@ -140,73 +130,55 @@ def test_dropin_install_is_reversible():
     assert L("ckpt").model("cpu", None) == "m" and L().processor() == "p"
 
 
-@needs_reference
 def test_reference_detection_predictor_config1_and_dropin_cpu():
     """BASELINE config 1: one 1024x1024 synthetic page (the reference's own conftest page) through the reference
-    DetectionPredictor on CPU — (a) with the reference's own model (plumbing check of the stock path), (b) with
-    B200EfficientViT over the oracle engine bound through surya_b200.dropin.  Same heatmaps -> same TextDetectionResult."""
-    from oracle import ref_predictors as RP
-    from surya_b200 import dropin
-    from surya_b200.config import det_default
-    from surya_b200.detection import B200EfficientViT
-    from surya_b200.synth import det_state_dict
-
-    RP.install_predictors()
-    from surya.detection import DetectionPredictor
-    from surya.detection.schema import TextDetectionResult
-
-    cfg = det_default()
-    sd = det_state_dict(cfg, seed=0)
-    ref_model = ref_shim.build_reference_det_model(cfg, sd)
-    proc = RP.synthetic_det_processor(1024)
-    page = RP.conftest_page(1024)
-
-    Stock = type("StockDetectionPredictor", (DetectionPredictor,), {"model_loader_cls": dropin.loader_for(ref_model, proc)})
-    stock = Stock(device="cpu", dtype=torch.float32)
-    stock.disable_tqdm = True
-    res_ref = stock([page])
-    assert len(res_ref) == 1 and isinstance(res_ref[0], TextDetectionResult)
-    assert res_ref[0].image_bbox == [0, 0, 1024, 1024]
-
-    pred = dropin.detection_predictor(B200EfficientViT(RP.OracleDetEngine(cfg, sd)), proc, device="cpu", dtype=torch.float32)
-    pred.disable_tqdm = True
-    res = pred([page], include_maps=False)
-    assert len(res) == 1 and res[0].image_bbox == [0, 0, 1024, 1024]
-    assert [b.polygon for b in res[0].bboxes] == [b.polygon for b in res_ref[0].bboxes]
-    # and the heat maps the two models hand to the post-processing are the same tensor up to fp32 noise
-    x = torch.from_numpy(proc(np.asarray(page, dtype=np.uint8))["pixel_values"][0])[None]
-    with torch.inference_mode():
-        a = ref_model(pixel_values=x).logits
-    b = B200EfficientViT(RP.OracleDetEngine(cfg, sd))(pixel_values=x).logits
-    assert (a - b).abs().max().item() < 1e-4
-
-
-@needs_reference
-def test_det_postprocess_oracle_pinned_to_reference():
-    """oracle.det_oracle.dynamic_thresholds / detect_boxes and the product's text_boxes_from_front against the reference's own
-    surya.detection.heatmap functions on synthetic heat maps (smooth blobs of text-line shape): identical thresholds, boxes and
-    confidences."""
-    import cv2
+    DetectionPredictor over its own model on CPU (tests/golden/reference_host.pt) against B200EfficientViT over the oracle engine:
+    the same segmentation logits (seeded sample) up to fp32 noise, and the same polygons from the product's host stages on the
+    heat map upsampled like the predictor does."""
+    import torch.nn.functional as F
 
     from oracle import det_oracle as D
     from oracle import ref_predictors as RP
+    from oracle.make_golden import array_digest
+    from surya_b200.config import det_default
+    from surya_b200.detection import B200EfficientViT, text_boxes_from_front
+    from surya_b200.pipeline import page_polygons
+    from surya_b200.synth import det_normalize, det_state_dict
+
+    g = torch.load(GOLDEN / "reference_host.pt")["det_config1"]
+    cfg = det_default()
+    sd = det_state_dict(cfg, seed=0)
+    page = np.asarray(RP.conftest_page(1024), dtype=np.uint8)
+    assert array_digest(page) == g["page_digest"], "the conftest page renders differently here"
+    assert g["image_bbox"] == [0, 0, 1024, 1024]
+    x = det_normalize(page[None])
+    logits = B200EfficientViT(RP.OracleDetEngine(cfg, sd))(pixel_values=x).logits.float()
+    assert tuple(logits.shape[1:]) == g["logits_shape"]
+    assert (logits[0].reshape(logits.shape[1], -1)[:, g["logit_index"]] - g["logits"]).abs().max().item() < 1e-4
+    heat = F.interpolate(logits, size=(1024, 1024), mode="bilinear", align_corners=False)[0, 0].numpy()
+    tt, low, _ = D.dynamic_thresholds(heat)
+    boxes, conf = text_boxes_from_front(heat, (heat > low).astype(np.uint8), float(tt), float(low))
+    polys, pconf = page_polygons(boxes, conf, (1024, 1024), (1024, 1024))
+    assert [[[float(v) for v in pt] for pt in p] for p in polys] == g["polygons"]
+    assert np.allclose(pconf, g["conf"], atol=1e-6)
+
+
+def test_det_postprocess_oracle_pinned_to_reference():
+    """oracle.det_oracle.dynamic_thresholds / detect_boxes and the product's text_boxes_from_front against what the reference's own
+    surya.detection.heatmap functions returned on the same synthetic heat maps (smooth blobs of text-line shape; stored in
+    tests/golden/reference_host.pt): identical thresholds, boxes and confidences."""
+    from oracle import det_oracle as D
+    from oracle.make_golden import array_digest, det_postprocess_maps
     from surya_b200.detection import text_boxes_from_front
 
-    RP.install_predictors()
-    from surya.detection.heatmap import detect_boxes, get_dynamic_thresholds
-
-    rng = np.random.default_rng(5)
-    for trial in range(3):
-        m = np.zeros((512, 640), np.float32)
-        for _ in range(25):
-            x, y = int(rng.integers(0, 560)), int(rng.integers(0, 480))
-            w, h = int(rng.integers(30, 200)), int(rng.integers(6, 24))
-            m[y:y + h, x:x + w] = rng.uniform(0.3, 1.0)
-        m = cv2.GaussianBlur(m, (0, 0), 2.0).astype(np.float16).astype(np.float32)     # 16-bit-valued like the engine's maps
-        tt_ref, low_ref = get_dynamic_thresholds(m, 0.6, 0.35)
+    golden = torch.load(GOLDEN / "reference_host.pt")["det_boxes"]
+    maps = det_postprocess_maps()
+    assert len(maps) == len(golden)
+    for m, ref in zip(maps, golden):
+        assert array_digest(m) == ref["map_digest"], "the synthetic heat map differs from the one the reference saw"
         tt, low, _ = D.dynamic_thresholds(m)
-        assert float(tt) == float(tt_ref) and float(low) == float(low_ref)
-        ref_boxes, ref_conf = detect_boxes(m, 0.6, 0.35)
+        assert (float(tt), float(low)) == ref["thresholds"]
+        ref_boxes, ref_conf = [b.numpy() for b in ref["boxes"]], ref["conf"].numpy()
         boxes, conf = D.detect_boxes(m)
         pboxes, pconf = text_boxes_from_front(m.astype(np.float16), (m > low).astype(np.uint8), float(tt), float(low))
         assert len(ref_boxes) == len(boxes) == len(pboxes) and len(boxes) > 3
@@ -215,48 +187,28 @@ def test_det_postprocess_oracle_pinned_to_reference():
         assert np.allclose(ref_conf, conf, atol=0) and np.allclose(ref_conf, pconf, atol=1e-7)
 
 
-@needs_reference
 def test_pipeline_host_stages_pinned_to_reference():
-    """surya_b200.pipeline.page_polygons / slice_polygon against the reference's get_and_clean_boxes + parallel_get_boxes expansion
-    (surya/detection/heatmap.py:125-175) and slice_polys_from_image (surya/input/processing.py:57-101) on synthetic heat maps."""
-    import cv2
-
+    """surya_b200.pipeline.page_polygons / slice_polygon against what the reference's get_and_clean_boxes + parallel_get_boxes
+    expansion (surya/detection/heatmap.py:125-175) and slice_polys_from_image (surya/input/processing.py:57-101) returned on the same
+    synthetic heat maps and pages (tests/golden/reference_host.pt; slices compared through sha256 digests of their bytes)."""
     from oracle import det_oracle as D
-    from oracle import ref_predictors as RP
+    from oracle.make_golden import array_digest, pipeline_host_cases
     from surya_b200.detection import text_boxes_from_front
     from surya_b200.pipeline import page_polygons, slice_polygon
 
-    RP.install_predictors()
-    from surya.detection.heatmap import get_and_clean_boxes
-    from surya.input.processing import slice_polys_from_image
-    from surya.settings import settings
-
-    rng = np.random.default_rng(9)
-    for trial in range(3):
-        H, W = 512, 640
-        m = np.zeros((H, W), np.float32)
-        for _ in range(20):
-            x, y = int(rng.integers(0, W - 60)), int(rng.integers(0, H - 30))
-            w, h = int(rng.integers(30, 220)), int(rng.integers(6, 30))
-            m[y:y + h, x:x + w] = rng.uniform(0.3, 1.0)
-        m[40:60, 100:300] = 0.9
-        m[44:56, 150:250] = 0.95                                   # a box contained in another one
-        m = cv2.GaussianBlur(m, (0, 0), 1.5).astype(np.float16).astype(np.float32)
-        img_size = (W * 2, H * 2) if trial == 1 else (W, H)       # also exercise the rescale path
-        ref = get_and_clean_boxes(m, [W, H], img_size)
-        for box in ref:
-            if box.height < 3 * box.width:
-                box.expand(x_margin=0, y_margin=settings.DETECTOR_BOX_Y_EXPAND_MARGIN)
-                box.fit_to_bounds([0, 0, img_size[0], img_size[1]])
+    golden = torch.load(GOLDEN / "reference_host.pt")["page_polys"]
+    cases = pipeline_host_cases()
+    assert len(cases) == len(golden)
+    for (m, img_size, page), ref in zip(cases, golden):
+        assert array_digest(m) == ref["map_digest"], "the synthetic heat map differs from the one the reference saw"
+        H, W = m.shape
         tt, low, _ = D.dynamic_thresholds(m)
         boxes, conf = text_boxes_from_front(m, (m > low).astype(np.uint8), float(tt), float(low))
         polys, pconf = page_polygons(boxes, conf, img_size, (W, H))
-        assert len(polys) == len(ref) and len(polys) > 3
-        for p, r, c in zip(polys, ref, pconf):
-            assert [[float(v) for v in pt] for pt in p] == [[float(v) for v in pt] for pt in r.polygon], (p, r.polygon)
-            assert abs(c - r.confidence) < 1e-6
-        if trial != 1:
-            page = rng.integers(0, 256, size=(H, W, 3)).astype(np.float32)
-            ref_slices = slice_polys_from_image(page, [[[int(v) for v in pt] for pt in r.polygon] for r in ref])
-            for p, rs in zip(polys, ref_slices):
-                assert np.array_equal(slice_polygon(page, p), rs)
+        assert len(polys) == len(ref["polygons"]) and len(polys) > 3
+        for p, r, c, rc in zip(polys, ref["polygons"], pconf, ref["conf"]):
+            assert [[float(v) for v in pt] for pt in p] == r, (p, r)
+            assert abs(c - rc) < 1e-6
+        assert (page is None) == (ref["slice_digests"] is None)
+        if page is not None:
+            assert [array_digest(slice_polygon(page, p)) for p in polys] == ref["slice_digests"]

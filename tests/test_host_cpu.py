@@ -377,8 +377,8 @@ def test_oracle_pinned_nonsquare_swin_and_cellpass_prompt():
     sde, sdd = swin_state_dict(enc_cfg, g["meta"]["seed"]), adetr_table_state_dict(cfg.decoder, g["meta"]["seed"])
     x = layout_synthetic_pages(2, enc_cfg.image_size, seed=g["meta"]["page_seed"])
     tok, done, enc, heads = L.table_greedy(sde, sdd, cfg, x, g["prompt"], g["meta"]["steps"])
-    assert enc.shape == g["encoder"].shape == (2, 128, 1024)
-    assert (enc - g["encoder"]).abs().max().item() < 1e-5
+    assert enc.shape == g["encoder_shape"] == (2, 128, 1024)
+    assert (enc.reshape(2 * 128, -1)[g["encoder_rows"]] - g["encoder"]).abs().max().item() < 1e-5
     for k, v in g["heads"].items():
         assert (heads[k] - v).abs().max().item() < 1e-4, k
     assert torch.equal(tok, g["tokens"])

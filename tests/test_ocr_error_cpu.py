@@ -3,7 +3,6 @@ written by oracle/make_golden.py), the host pack plan, and the op sequence of su
 for the C-ABI ops (wiring / index check only — the kernels themselves are compared on the GPU in test_ocr_error_gpu.py)."""
 import math
 from pathlib import Path
-from types import SimpleNamespace
 
 import numpy as np
 import pytest
@@ -11,14 +10,12 @@ import torch
 import torch.nn.functional as F
 
 from oracle import ocr_error_oracle as E
-from oracle import ref_shim
 from surya_b200 import _lib
 from surya_b200 import ocr_error as OE
 from surya_b200.config import ocr_error_default, ocr_error_tiny
 from surya_b200.synth import ocr_error_state_dict, ocr_error_synthetic_batch
 
 GOLDEN = Path(__file__).parent / "golden"
-needs_reference = pytest.mark.skipif(not ref_shim.available(), reason="/root/reference is only mounted in the build container")
 
 
 @pytest.mark.parametrize("kind", ["tiny", "default"])
@@ -128,57 +125,22 @@ def _unpack(plan, cfg):
     return torch.from_numpy(ids), torch.from_numpy(mask)
 
 
-class _HashTokenizer:
-    """Stand-in for DistilBertTokenizer's call (surya/ocr_error/__init__.py:28-30): words hashed into the vocabulary, [CLS]-like id
-    first, padding='longest' on the right.  (The real tokenizer needs the checkpoint's vocab file; it is host string code.)"""
-
-    def __init__(self, cfg):
-        self.cfg = cfg
-
-    def __call__(self, texts, padding="longest", truncation=True, return_tensors="pt"):
-        import zlib
-        rows = [[101 % self.cfg.vocab_size] + [1 + zlib.crc32(w.encode()) % (self.cfg.vocab_size - 1) for w in t.split()] for t in texts]
-        L = min(max(len(r) for r in rows), self.cfg.max_position_embeddings)
-        ids = torch.full((len(rows), L), self.cfg.pad_token_id, dtype=torch.int64)
-        mask = torch.zeros((len(rows), L), dtype=torch.int64)
-        for i, r in enumerate(rows):
-            r = r[:L]
-            ids[i, :len(r)] = torch.tensor(r)
-            mask[i, :len(r)] = 1
-        return SimpleNamespace(input_ids=ids, attention_mask=mask)
-
-
-@needs_reference
 def test_reference_ocr_error_predictor_dropin_cpu():
-    """The reference's UNMODIFIED OCRErrorPredictor (a) over its own DistilBertForSequenceClassification and (b) over the
-    B200DistilBert mirror bound through surya_b200.dropin (the network behind the mirror is the CPU oracle here: no GPU in this
-    container) — same labels for the same texts, batches of 3 with a ragged tail."""
-    from surya_b200 import dropin
+    """Labels of the reference's UNMODIFIED OCRErrorPredictor over its own DistilBertForSequenceClassification (stored in
+    tests/golden/reference_host.pt by oracle/make_golden.py) against surya_b200.ocr_error.detect_errors over the B200DistilBert
+    mirror for the same texts, batches of 3 with a ragged tail (the network behind the mirror is the CPU oracle here)."""
+    from oracle.make_golden import ocr_error_texts
 
-    ref_shim.install()
-    from surya.ocr_error import OCRErrorPredictor
-    from surya.ocr_error.schema import OCRErrorDetectionResult
-
+    g = torch.load(GOLDEN / "reference_host.pt")["ocr_error"]
     cfg = ocr_error_tiny()
     sd = ocr_error_state_dict(cfg, seed=0)
-    rng = np.random.default_rng(0)
-    words = [f"w{i}" for i in range(300)]
-    texts = [" ".join(rng.choice(words, size=int(rng.integers(2, 30)))) for _ in range(8)]
-    tok = _HashTokenizer(cfg)
-
-    ref_model = ref_shim.build_reference_ocr_error_model(cfg, sd)
-    Stock = type("StockOCRErrorPredictor", (OCRErrorPredictor,), {"model_loader_cls": dropin.loader_for(ref_model, tok)})
-    stock = Stock(device="cpu", dtype=torch.float32)
-    stock.disable_tqdm = True
-    res_ref = stock(texts, batch_size=3)
-    assert isinstance(res_ref, OCRErrorDetectionResult) and len(res_ref.labels) == len(texts)
-
+    texts = ocr_error_texts()
+    assert texts == g["texts"]
     mirror = object.__new__(OE.B200DistilBert)
     mirror.config = mirror.cfg = cfg
     mirror.dtype, mirror.device = torch.float32, torch.device("cpu")
     mirror.forward_packed = lambda plan: E.forward(sd, cfg, *_unpack(plan, cfg))
-    pred = dropin.ocr_error_predictor(mirror, tok, device="cpu", dtype=torch.float32)
-    pred.disable_tqdm = True
-    res = pred(texts, batch_size=3)
-    assert res.labels == res_ref.labels and res.texts == texts
-    assert len(set(res.labels)) == 2, res.labels
+    tok = E.HashTokenizer(cfg)(texts)
+    labels = OE.detect_errors(mirror, tok.input_ids, tok.attention_mask, batch_size=g["batch_size"])
+    assert labels == g["labels"]
+    assert len(set(labels)) == 2, labels

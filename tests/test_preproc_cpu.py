@@ -1,8 +1,11 @@
 """Recognition crop preprocessing (SURVEY §8 f2), CPU side: the numpy restatement of OpenCV's float32 Lanczos4 / cubic resize is pinned
 against cv2 itself (the reference's dependency), the whole per-crop chain against the product's cv2-based host mirror (itself pinned to
 the reference processor in test_host_cpu.py::test_tiling_and_prompt_match_oracle), and the host plan of the device path is checked."""
+from pathlib import Path
+
 import numpy as np
 import pytest
+import torch
 
 cv2 = pytest.importorskip("cv2")
 
@@ -10,6 +13,7 @@ from oracle import preproc_oracle as P
 from surya_b200.config import tiny_rec
 from surya_b200.recognition import build_preprocess_plan, scale_to_fit, tile_image
 
+GOLDEN = Path(__file__).resolve().parent / "golden"
 TOL_255 = 5e-4          # on the 0..255 scale: float32 summation-order noise of a 64-tap sum of values up to 255 (measured ~1e-4)
 
 
@@ -58,21 +62,21 @@ def test_preprocess_plan():
 
 
 def test_crop_chain_pinned_to_the_reference_processor():
-    """The restatement against the reference's OWN SuryaOCRProcessor (scale_to_fit + _process_and_tile, imported unmodified from
-    /root/reference; skipped where it is not mounted): same grids, tiles equal to float32 rounding of the OpenCV resizes."""
-    from oracle import ref_shim
-    if not ref_shim.available():
-        pytest.skip("/root/reference is only mounted in the build container")
-    from oracle import ref_predictors as RP
+    """The restatement against what the reference's OWN SuryaOCRProcessor (scale_to_fit + _process_and_tile, unmodified) returned
+    for the same seeded crops (tests/golden/reference_host.pt, written by oracle/make_golden.py): same grids, tiles equal to float32
+    rounding of the OpenCV resizes — a seeded sample of tile rows element by element, every row through its sum and sum of squares."""
+    from oracle.make_golden import preproc_crops
 
-    RP.install_predictors()
     cfg = tiny_rec()
-    proc = RP.synthetic_ocr_processor(cfg)
-    rng = np.random.default_rng(11)
-    for h, w in ((48, 512), (40, 300), (300, 2000), (20, 60), (56, 560), (97, 1403)):
-        crop = rng.integers(0, 256, (h, w, 3), dtype=np.uint8)
-        img = proc.scale_to_fit(np.asarray(crop, dtype=np.float32), (1024, 256))
-        ref_tiles, ref_grid = proc._process_and_tile(img)
+    golden = torch.load(GOLDEN / "reference_host.pt")["crop_chain"]
+    crops = preproc_crops()
+    assert len(crops) == len(golden)
+    tol = 2 * TOL_255 / 255 / 0.224
+    for crop, ref in zip(crops, golden):
         tiles, grid = P.process_crop(crop, cfg.vision_encoder.patch_size, cfg.merge_size)
-        assert tuple(int(g) for g in ref_grid) == tuple(grid)
-        assert np.abs(tiles - ref_tiles.numpy()).max() <= 2 * TOL_255 / 255 / 0.224, (h, w)
+        assert crop.shape == ref["shape"] and tuple(grid) == ref["grid"], crop.shape
+        assert tiles.shape[0] == ref["row_sums"].numel()
+        assert np.abs(tiles[ref["rows"].numpy()] - ref["tile_rows"].numpy()).max() <= tol, crop.shape
+        assert np.abs(tiles.astype(np.float64).sum(1) - ref["row_sums"].numpy()).max() <= tol * tiles.shape[1], crop.shape
+        sq_tol = tol * (2 * np.abs(tiles.astype(np.float64)).sum(1) + tol * tiles.shape[1])     # |a^2 - b^2| <= |a - b| (2|a| + |a - b|)
+        assert (np.abs((tiles.astype(np.float64) ** 2).sum(1) - ref["row_sq"].numpy()) <= sq_tol).all(), crop.shape

@@ -62,29 +62,6 @@ int sb_gemm_argmax_tile(int M, int N);
 /* rs[row] = rsqrt(mean(x[row]^2) + eps) in the summation order sb_gemm_rmsnorm's in-kernel pass uses (bit-identical). */
 int sb_row_rstd(int dtype, const void* x, int ldx, float* rs, int rows, int H, float eps, const int* src_rows, void* stream);
 
-/* A chain of up to 4 dependent nn.Linear calls on <= 256 rows in ONE persistent launch (grid-wide barrier between phases): the
- * o_proj -> gate/up -> down -> next-layer qkv sequence of a Qwen2DecoderLayer at q_len = 1 (decoder/__init__.py:288-310), where
- * every Linear needs the complete rows of its predecessor.  Phase semantics are sb_gemm's (rms_eps > 0: sb_gemm_rmsnorm's
- * in-kernel folded norm); results are bit-identical to separate launches with the same tile width (force_bn, 0 = sb_gemm_chain_bn).
- * barrier: 3 zero-initialised uint32 in device memory owned by the caller ([2] != 0 after a launch = barrier timeout). */
-typedef struct {
-  const void* A; int lda;
-  const void* W; int ldw;
-  void* C; int ldc;
-  int M, N, K;
-  const float* bias;
-  const void* residual; int ldr;
-  int act, swiglu;
-  float rms_eps;
-  int force_bn;
-} sb_gemm_phase;
-int sb_gemm_chain(int dtype, const sb_gemm_phase* phases, int n_phases, unsigned int* barrier, void* stream);
-int sb_gemm_chain_bn(int M, int N, int swiglu);
-/* sb_gemm_chain with a timeline of CTA 0 (globaltimer ns): timeline_dev[8 * phase + {0 phase start, 1 first k-block landed,
- * 2 last MMA issued, 3 accumulator ready, 4 epilogue done, 5 grid barrier passed}]; profiling aid. */
-int sb_gemm_chain_timeline(int dtype, const sb_gemm_phase* phases, int n_phases, unsigned int* barrier,
-                           unsigned long long* timeline_dev, void* stream);
-
 /* sb_gemm with an in-kernel timeline of CTA 0 (globaltimer ns into timeline_dev[0..42]); profiling aid. */
 int sb_gemm_timeline(int dtype, const void* A, int lda, const void* W, int ldw, void* C, int ldc, int M, int N, int K,
                      const float* bias, const void* residual, int ldr, int act, int swiglu, int force_bn,
@@ -218,11 +195,6 @@ int sb_rec_decode(sb_rec_engine* eng, const long long* input_ids, const int* slo
 int sb_rec_decode_steps(sb_rec_engine* eng, long long* ids_io, const int* slot, int* pos_io, int batch, int n_steps,
                         long long* tok_hist, float* score_hist, long long* bbox_hist, unsigned char* done_hist,
                         int use_graph, void* stream);
-
-/* Engine switches.  "chain" (0/1, default 0 or $SB_CHAIN): run o_proj -> gate/up -> down -> next-layer qkv of every decoder layer
- * as one persistent sb_gemm_chain launch instead of four launches (same results up to the down projection's fp32 summation order:
- * the separate path uses the split-K kernel for it). */
-int sb_rec_set_option(sb_rec_engine* eng, const char* name, int value);
 
 /* Recognition crop preprocessing on the device (SURVEY §8 f2): SuryaOCRProcessor.scale_to_fit (cv2 INTER_LANCZOS4 when the pixel
  * count is outside [168*168, 1024*256], surya/common/surya/processor/__init__.py:140-178) + _process_and_tile (cv2 INTER_CUBIC to the

@@ -13,8 +13,6 @@
 #include "ops.cuh"
 #include "sb_ptx.cuh"
 
-#include <cstdlib>
-
 namespace sb {
 
 template <typename T> struct Mma;
@@ -427,228 +425,8 @@ __global__ void __launch_bounds__(128) decode_attn_kernel(const DecodeKParams p)
   }
 }
 
-// ------------------------------------------------------------------------------------------- decode attention, version 2
-// Same contract and rounding points as decode_attn_kernel; the memory round trips overlap instead of following each other:
-//   t = 0   the V rows already in the cache ([0, pos) x HD, one contiguous block per (slot, kv head)) start moving into shared
-//           memory with ONE cp.async.bulk (TMA 1-D, mbarrier completion);
-//           every thread requests the K row of "its" key into registers (one key per thread for up to 160 keys);
-//           the q / k / v slices of this row's fused qkv are requested.
-//   then    RoPE (q heads + new key) and the cache append, scores from the K registers, softmax, and P.V out of shared memory.
-// Round 1's kernel did these as three dependent phases (q/k row -> K -> V, the last one in up to three dependent batches):
-// 9 / 15 / 21 us at 46 / 110 / 173 cached tokens (profiles/r02_decode_parts.md).
-template <typename T, int HD, int G>
-__global__ void __launch_bounds__(160) decode_attn_v2_kernel(const DecodeKParams p) {
-  constexpr int NT = 160, HALF = HD / 2, VPR = HD / 8;
-  extern __shared__ __align__(128) uint8_t smem_dec2[];
-  T* v_s = reinterpret_cast<T*>(smem_dec2);                                   // [s_max][HD]
-  float* sc = reinterpret_cast<float*>(smem_dec2 + static_cast<size_t>(p.s_max) * HD * sizeof(T));   // [G][s_max]
-  float* q_s = sc + G * p.s_max;                                              // [G][HD]
-  float* part = q_s + G * HD;                                                 // [2][G][HD] P.V partials of the two key halves
-  __shared__ float s_red[5][G];
-  __shared__ float s_max_g[G], s_sum_g[G];
-  __shared__ __align__(8) uint64_t vbar;
-
-  pdl_trigger();
-  const int tid = threadIdx.x, warp = tid >> 5, lane = tid & 31;
-  if (tid == 0) {
-    mbar_init(&vbar, 1);
-    mbar_fence_init();
-  }
-  pdl_wait();
-  const int b = blockIdx.x, kvh = blockIdx.y;
-  const int slot = p.slot[b];
-  const int pos = p.pos[b];
-  T* orow0 = reinterpret_cast<T*>(p.out) + static_cast<size_t>(b) * p.ldo + (kvh * G) * HD;
-  if (pos < 0 || pos >= p.s_max) {      // full slot: never write past it (host callers reject this before launching)
-    for (int i = tid; i < G * HD; i += NT) orow0[i] = from_f<T>(0.f);
-    return;
-  }
-  const int n_keys = pos + 1;
-  const T* row = reinterpret_cast<const T*>(p.qkv) + static_cast<size_t>(b) * p.ld;
-  T* kc = reinterpret_cast<T*>(p.kcache) + (static_cast<size_t>(slot) * p.n_kv_heads + kvh) * p.s_max * HD;
-  T* vc = reinterpret_cast<T*>(p.vcache) + (static_cast<size_t>(slot) * p.n_kv_heads + kvh) * p.s_max * HD;
-  __syncthreads();                       // barrier initialised
-  const uint32_t v_bytes = static_cast<uint32_t>(pos) * HD * sizeof(T);
-  if (tid == 0 && pos > 0) {
-    mbar_expect_tx(&vbar, v_bytes);
-    asm volatile("cp.async.bulk.shared::cluster.global.mbarrier::complete_tx::bytes [%0], [%1], %2, [%3];" ::"r"(smem_u32(v_s)),
-                 "l"(reinterpret_cast<uint64_t>(vc)), "r"(v_bytes), "r"(smem_u32(&vbar))
-                 : "memory");
-  }
-  // this thread's first key (cached rows only: row `pos` is produced below)
-  uint4 kreg[VPR];
-  const bool have_k = tid < pos;
-  if (have_k) {
-    const uint4* kr = reinterpret_cast<const uint4*>(kc + static_cast<size_t>(tid) * HD);
-#pragma unroll
-    for (int c = 0; c < VPR; ++c) kreg[c] = kr[c];
-  }
-  // ---- RoPE on the G query heads and the new key; append k, v (global cache + shared V tile)
-  for (int idx = tid; idx < (G + 1) * HALF; idx += NT) {
-    const int hh = idx / HALF, i = idx % HALF;
-    const T* src = (hh < G) ? row + (kvh * G + hh) * HD : row + (p.n_heads + kvh) * HD;
-    const float f = static_cast<float>(pos) * p.inv_freq[i];
-    const float c = rnd<T>(cosf(f)), sn = rnd<T>(sinf(f));
-    const float x1 = to_f<T>(src[i]), x2 = to_f<T>(src[i + HALF]);
-    const float o1 = rnd<T>(rnd<T>(x1 * c) + rnd<T>(-x2 * sn));
-    const float o2 = rnd<T>(rnd<T>(x2 * c) + rnd<T>(x1 * sn));
-    if (hh < G) {
-      q_s[hh * HD + i] = o1;
-      q_s[hh * HD + i + HALF] = o2;
-    } else {
-      kc[static_cast<size_t>(pos) * HD + i] = from_f<T>(o1);
-      kc[static_cast<size_t>(pos) * HD + i + HALF] = from_f<T>(o2);
-      sc[i] = o1;                        // the new key, parked in the (not yet used) score area for the dot product below
-      sc[i + HALF] = o2;
-    }
-  }
-  {
-    const T* vsrc = row + (p.n_heads + p.n_kv_heads + kvh) * HD;
-    for (int i = tid; i < HD; i += NT) {
-      const T vv = vsrc[i];
-      vc[static_cast<size_t>(pos) * HD + i] = vv;
-      v_s[static_cast<size_t>(pos) * HD + i] = vv;
-    }
-  }
-  __syncthreads();
-  // ---- score of the new key (one warp per group of query heads), then of the cached keys
-  float newk_dot[G];
-  if (warp == 0) {
-#pragma unroll
-    for (int gq = 0; gq < G; ++gq) {
-      float a = 0.f;
-      for (int i = lane; i < HD; i += 32) a += q_s[gq * HD + i] * sc[i];
-      newk_dot[gq] = warp_sum(a);
-    }
-  }
-  __syncthreads();                       // everybody is done reading the parked key
-  float tmax[G];
-#pragma unroll
-  for (int gq = 0; gq < G; ++gq) tmax[gq] = -INFINITY;
-  if (warp == 0 && lane == 0) {
-#pragma unroll
-    for (int gq = 0; gq < G; ++gq) {
-      const float sv = newk_dot[gq] * p.scale;
-      sc[gq * p.s_max + pos] = sv;
-      tmax[gq] = sv;
-    }
-  }
-  for (int j = tid; j < pos; j += NT) {
-    if (j != tid) {                       // keys beyond the first NT: plain (dependent) loads, rare
-      const uint4* kr = reinterpret_cast<const uint4*>(kc + static_cast<size_t>(j) * HD);
-#pragma unroll
-      for (int c = 0; c < VPR; ++c) kreg[c] = kr[c];
-    }
-    float acc[G];
-#pragma unroll
-    for (int gq = 0; gq < G; ++gq) acc[gq] = 0.f;
-#pragma unroll
-    for (int c = 0; c < VPR; ++c) {
-      const T* e = reinterpret_cast<const T*>(&kreg[c]);
-#pragma unroll
-      for (int x = 0; x < 8; ++x) {
-        const float kf = to_f<T>(e[x]);
-#pragma unroll
-        for (int gq = 0; gq < G; ++gq) acc[gq] += q_s[gq * HD + c * 8 + x] * kf;
-      }
-    }
-#pragma unroll
-    for (int gq = 0; gq < G; ++gq) {
-      const float sv = acc[gq] * p.scale;
-      sc[gq * p.s_max + j] = sv;
-      tmax[gq] = fmaxf(tmax[gq], sv);
-    }
-  }
-#pragma unroll
-  for (int gq = 0; gq < G; ++gq) {
-    const float m = warp_max(tmax[gq]);
-    if (lane == 0) s_red[warp][gq] = m;
-  }
-  __syncthreads();
-  if (tid < G) s_max_g[tid] = fmaxf(fmaxf(fmaxf(s_red[0][tid], s_red[1][tid]), fmaxf(s_red[2][tid], s_red[3][tid])), s_red[4][tid]);
-  __syncthreads();
-  float tsum[G];
-#pragma unroll
-  for (int gq = 0; gq < G; ++gq) tsum[gq] = 0.f;
-  for (int j = tid; j < n_keys; j += NT) {
-#pragma unroll
-    for (int gq = 0; gq < G; ++gq) {
-      const float pv = __expf(sc[gq * p.s_max + j] - s_max_g[gq]);
-      tsum[gq] += pv;
-      sc[gq * p.s_max + j] = rnd<T>(pv);
-    }
-  }
-#pragma unroll
-  for (int gq = 0; gq < G; ++gq) {
-    const float sm = warp_sum(tsum[gq]);
-    if (lane == 0) s_red[warp][gq] = sm;
-  }
-  __syncthreads();
-  if (tid < G) s_sum_g[tid] = s_red[0][tid] + s_red[1][tid] + s_red[2][tid] + s_red[3][tid] + s_red[4][tid];
-  // ---- O = P V out of shared memory: thread = (key parity, dim); every thread walks its half of the keys
-  if (pos > 0) mbar_wait(&vbar, 0);
-  __syncthreads();
-  {
-    const int par = tid / HD, d = tid % HD;            // NT = 2 * 80 for HD = 80; for other HD see the loop bounds below
-    if (par < 2 && tid < 2 * HD) {
-      float acc[G];
-#pragma unroll
-      for (int gq = 0; gq < G; ++gq) acc[gq] = 0.f;
-      for (int j = par; j < n_keys; j += 2) {
-        const float vf = to_f<T>(v_s[static_cast<size_t>(j) * HD + d]);
-#pragma unroll
-        for (int gq = 0; gq < G; ++gq) acc[gq] += sc[gq * p.s_max + j] * vf;
-      }
-#pragma unroll
-      for (int gq = 0; gq < G; ++gq) part[(par * G + gq) * HD + d] = acc[gq];
-    }
-  }
-  __syncthreads();
-  for (int i = tid; i < G * HD; i += NT) {
-    const float o = part[i] + part[G * HD + i];
-    orow0[i] = from_f<T>(o / s_sum_g[i / HD]);
-  }
-}
-
-template <typename T, int HD, int G>
-static int launch_decode_v2(const DecodeAttnArgs& a, cudaStream_t st) {
-  const size_t smem = static_cast<size_t>(a.s_max) * HD * sizeof(T) + (static_cast<size_t>(G) * a.s_max + 3 * G * HD) * sizeof(float);
-  auto kern = decode_attn_v2_kernel<T, HD, G>;
-  static size_t attr = 0;
-  if (smem > 48 * 1024 && smem > attr) {
-    if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)smem) != cudaSuccess) {
-      cudaGetLastError();
-      return -100;                       // does not fit: the caller falls back to the streaming kernel
-    }
-    attr = smem;
-  }
-  DecodeKParams p;
-  p.qkv = a.qkv; p.ld = a.ld; p.kcache = a.kcache; p.vcache = a.vcache; p.slot = a.slot; p.pos = a.pos;
-  p.inv_freq = a.inv_freq; p.out = a.out; p.ldo = a.ldo;
-  p.n_heads = a.n_heads; p.n_kv_heads = a.n_kv_heads; p.s_max = a.s_max; p.scale = a.scale;
-  dim3 grid(a.batch, a.n_kv_heads), block(160);
-  launch_pdl(kern, grid, block, smem, st, p);
-  return launch_ok();
-}
-
-// OFF by default: measured 14 / 21 / 29 us against 9 / 15 / 21 us for the streaming kernel at 46 / 110 / 173 cached tokens
-// (B = 256, 4 kv heads): the 49 KB V tile allows 4 CTAs per SM instead of 10, the 1024 CTAs run in two lock-step waves and the
-// memory phase of a wave no longer overlaps anybody's arithmetic.  $SB_DECODE_ATTN_V2=1 enables it (tests cover both).
-static bool decode_v2_enabled() {
-  static int v = -1;
-  if (v < 0) { const char* e = getenv("SB_DECODE_ATTN_V2"); v = (e && e[0] == '1') ? 1 : 0; }
-  return v == 1;
-}
-
 template <typename T, int HD, int G>
 static int launch_decode(const DecodeAttnArgs& a, cudaStream_t st) {
-  // version 2 keeps the whole V tile of a (row, kv head) in shared memory: use it while that still leaves several CTAs per SM
-  if (HD <= 80 && decode_v2_enabled() &&
-      static_cast<size_t>(a.s_max) * HD * sizeof(T) + (static_cast<size_t>(G) * a.s_max + 3 * G * HD) * sizeof(float) <= 100 * 1024 &&
-      (static_cast<size_t>(a.s_max) * HD * sizeof(T)) % 16 == 0 && G * a.s_max >= HD) {
-    const int rc = launch_decode_v2<T, HD, G>(a, st);
-    if (rc != -100) return rc;
-  }
   constexpr int NKG = 128 / (HD / 8);
   size_t smem = (static_cast<size_t>(G) * HD + static_cast<size_t>(NKG) * G * HD + static_cast<size_t>(G) * a.s_max) *
                 sizeof(float);

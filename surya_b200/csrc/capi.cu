@@ -39,35 +39,6 @@ int sb_gemm_rmsnorm(int dtype, const void* A, int lda, const void* W, int ldw, v
 
 int sb_gemm_argmax_tile(int M, int N) { return gemm_argmax_tile(M, N); }
 
-static int chain_common(int dtype, const sb_gemm_phase* phases, int n_phases, unsigned int* barrier, unsigned long long* dbg,
-                        void* stream);
-
-int sb_gemm_chain(int dtype, const sb_gemm_phase* phases, int n_phases, unsigned int* barrier, void* stream) {
-  return chain_common(dtype, phases, n_phases, barrier, nullptr, stream);
-}
-
-int sb_gemm_chain_timeline(int dtype, const sb_gemm_phase* phases, int n_phases, unsigned int* barrier,
-                           unsigned long long* timeline_dev, void* stream) {
-  return chain_common(dtype, phases, n_phases, barrier, timeline_dev, stream);
-}
-
-static int chain_common(int dtype, const sb_gemm_phase* phases, int n_phases, unsigned int* barrier, unsigned long long* dbg,
-                        void* stream) {
-  if (!phases || n_phases < 1 || n_phases > 4) { set_error("sb_gemm_chain: 1..4 phases"); return -1; }
-  GemmArgs a[4];
-  a[0].dbg = dbg;
-  for (int i = 0; i < n_phases; ++i) {
-    const sb_gemm_phase& q = phases[i];
-    a[i].dtype = dtype; a[i].A = q.A; a[i].lda = q.lda; a[i].W = q.W; a[i].ldw = q.ldw; a[i].C = q.C; a[i].ldc = q.ldc;
-    a[i].M = q.M; a[i].N = q.N; a[i].K = q.K; a[i].bias = q.bias; a[i].residual = q.residual; a[i].ldr = q.ldr;
-    a[i].act = q.act; a[i].swiglu = q.swiglu; a[i].force_bn = q.force_bn;
-    if (q.rms_eps > 0.f) { a[i].ssq_inline = 1; a[i].ssq_eps = q.rms_eps; a[i].ssq_k = q.K; }
-  }
-  return gemm_chain_launch(a, n_phases, barrier, static_cast<cudaStream_t>(stream));
-}
-
-int sb_gemm_chain_bn(int M, int N, int swiglu) { return gemm_chain_bn(M, N, swiglu); }
-
 int sb_row_rstd(int dtype, const void* x, int ldx, float* rs, int rows, int H, float eps, const int* src_rows, void* stream) {
   return row_rstd(dtype, x, ldx, rs, rows, H, eps, src_rows, static_cast<cudaStream_t>(stream));
 }

@@ -37,19 +37,15 @@ struct FmbParams {
   void* out;              // NHWC [n_img, Ho, Wo, Cout]
 };
 
-template <typename T, int BKC, int COUT, int STAGES, int NW2>
+template <typename T, int COUT, int STAGES, int NW2>
 __global__ void __launch_bounds__(512, 1)
 fmb_fused_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_w1,
                  const __grid_constant__ CUtensorMap tma_w2, const FmbParams fp) {
   constexpr int BM = 128, TW = 16, TH = 8, CH = 128;                 // mid-channel chunk
-  // Cin = 32 (BKC == 32): the nine tap tiles of a pixel tile stay RESIDENT for all mid-channel chunks (one 64-byte-row TMA box each per
-  // tile instead of one per chunk) and W1 is streamed in [128 x 64] boxes that span a PAIR of taps (128-byte rows), which cuts the
-  // TMA line count per tile from 9216 to 3456 — the first version of this block was bound by the TMA engine, not by the tensor pipe.
-  constexpr bool RES_A = (BKC == 32);
+  constexpr int BKC = 64;                                            // input channels per GEMM1 k-block
   constexpr uint32_t A1_BYTES = BM * BKC * 2;
-  constexpr uint32_t W1_BYTES = RES_A ? CH * 64 * 2 : CH * BKC * 2;
-  constexpr uint32_t S1_BYTES = RES_A ? W1_BYTES : A1_BYTES + W1_BYTES;
-  constexpr uint32_t RESA_BYTES = RES_A ? 9 * A1_BYTES : 0;
+  constexpr uint32_t W1_BYTES = CH * BKC * 2;
+  constexpr uint32_t S1_BYTES = A1_BYTES + W1_BYTES;
   constexpr uint32_t A2_KB_BYTES = BM * 64 * 2;                      // one 64-channel k-block of the A2 tile (16 KB)
   constexpr uint32_t A2_BYTES = 2 * A2_KB_BYTES;                     // 128 mid channels
   constexpr uint32_t W2_KB_BYTES = COUT * 64 * 2, W2_BYTES = 2 * W2_KB_BYTES;
@@ -57,8 +53,7 @@ fmb_fused_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
 
   extern __shared__ uint8_t smem_raw[];
   uint8_t* smem = smem_raw + ((1024u - (smem_u32(smem_raw) & 1023u)) & 1023u);   // array + offset keeps the shared address space (STS / LDS, not generic ST / LD)
-  uint8_t* s_ra = smem;                                             // resident tap tiles (Cin = 32 only)
-  uint8_t* s_1 = s_ra + RESA_BYTES;
+  uint8_t* s_1 = smem;
   uint8_t* s_a2 = s_1 + STAGES * S1_BYTES;
   uint8_t* s_w2 = s_a2 + 2 * A2_BYTES;
   float* s_b1 = reinterpret_cast<float*>(s_w2 + NW2 * W2_BYTES);
@@ -74,9 +69,7 @@ fmb_fused_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
   uint64_t* w2_empty = w2_full + NW2;
   uint64_t* t2_full = w2_empty + NW2;
   uint64_t* t2_empty = t2_full + 1;
-  uint64_t* ra_full = t2_empty + 1;                                  // [9] resident tap tiles
-  uint64_t* ra_empty = ra_full + 9;
-  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(ra_empty + 9);
+  uint32_t* tmem_slot = reinterpret_cast<uint32_t*>(t2_empty + 1);
 
   const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
   const int tiles_per_img = fp.tiles_x * fp.tiles_y;
@@ -94,7 +87,6 @@ fmb_fused_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
     }
     for (int i = 0; i < NW2; ++i) { mbar_init(&w2_full[i], 1); mbar_init(&w2_empty[i], 1); }
     mbar_init(t2_full, 1); mbar_init(t2_empty, 4);
-    for (int i = 0; i < 9; ++i) { mbar_init(&ra_full[i], 1); mbar_init(&ra_empty[i], 1); }
     mbar_fence_init();
   }
   if (warp == 2) tmem_alloc(tmem_slot, TMEM_COLS);
@@ -115,7 +107,7 @@ fmb_fused_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
   if (warp == 0) {
     // ------------------------------------------------------------------ TMA producer
     if (lane == 0) {
-      int s = 0; uint32_t ph = 0; int wb = 0; uint32_t wph = 0; uint32_t raph = 0;
+      int s = 0; uint32_t ph = 0; int wb = 0; uint32_t wph = 0;
       auto load_w2 = [&](int j) {
         mbar_wait(&w2_empty[wb], wph ^ 1);
         mbar_expect_tx(&w2_full[wb], W2_BYTES);
@@ -128,21 +120,6 @@ fmb_fused_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
         coords(tile, img, oy0, ox0);
         const int x0 = ox0 * fp.stride - 1, y0 = oy0 * fp.stride - 1;
         for (int j = 0; j < nch; ++j) {
-          if constexpr (RES_A) {
-            for (int pr = 0; pr < 5; ++pr) {                          // tap pairs (0,1) (2,3) (4,5) (6,7) (8,-)
-              if (j == 0) {
-                for (int t = 2 * pr; t < 2 * pr + 2 && t < 9; ++t) {
-                  mbar_wait(&ra_empty[t], raph ^ 1);
-                  mbar_expect_tx(&ra_full[t], A1_BYTES);
-                  tma_load_4d(s_ra + t * A1_BYTES, &tma_a, &ra_full[t], 0, x0 + t % 3, y0 + t / 3, img);
-                }
-              }
-              mbar_wait(&s1_empty[s], ph ^ 1);
-              mbar_expect_tx(&s1_full[s], W1_BYTES);
-              tma_load_2d(s_1 + s * S1_BYTES, &tma_w1, &s1_full[s], pr * 64, j * CH);   // columns >= 288 are zero filled
-              if (++s == STAGES) { s = 0; ph ^= 1; }
-            }
-          } else {
           int kcol = 0;
           for (int r = 0; r < 3; ++r)
             for (int sx = 0; sx < 3; ++sx)
@@ -154,11 +131,9 @@ fmb_fused_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
                 tma_load_2d(sa + A1_BYTES, &tma_w1, &s1_full[s], kcol, j * CH);
                 if (++s == STAGES) { s = 0; ph ^= 1; }
               }
-          }
           if (j >= 1) load_w2(j - 1);
         }
         load_w2(nch - 1);
-        raph ^= 1;
       }
     }
   } else if (warp == 1) {
@@ -166,7 +141,7 @@ fmb_fused_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
     if (lane == 0) {
       constexpr uint32_t idesc1 = umma_idesc_f16(TypeInfo<T>::umma_fmt, BM, CH);
       constexpr uint32_t idesc2 = umma_idesc_f16(TypeInfo<T>::umma_fmt, BM, COUT);
-      int s = 0; uint32_t ph = 0; int wb = 0; uint32_t wph = 0; uint32_t raph = 0;
+      int s = 0; uint32_t ph = 0; int wb = 0; uint32_t wph = 0;
       uint32_t t1ph[2] = {0, 0}, a2ph[2] = {0, 0}, t2ph = 0;
       auto gemm2 = [&](int j) {
         const int b = j & 1;
@@ -194,33 +169,16 @@ fmb_fused_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
           t1ph[b] ^= 1;
           tc_fence_after();
           const uint32_t d1 = tmem_base + b * CH;
-          if constexpr (RES_A) {
-            for (int pr = 0; pr < 5; ++pr) {
-              mbar_wait(&s1_full[s], ph);
-              tc_fence_after();
-              const uint64_t dbp = umma_desc_k128(smem_u32(s_1 + s * S1_BYTES));     // [128 x 64]: taps 2pr (cols 0..31), 2pr+1 (32..63)
-              for (int t = 2 * pr; t < 2 * pr + 2 && t < 9; ++t) {
-                if (j == 0) { mbar_wait(&ra_full[t], raph); tc_fence_after(); }
-                const uint64_t da = umma_desc_k64(smem_u32(s_ra + t * A1_BYTES));
-#pragma unroll
-                for (int k = 0; k < 2; ++k) umma_f16(d1, da + 2 * k, dbp + 4 * (t & 1) + 2 * k, idesc1, (t | k) != 0 ? 1u : 0u);
-                if (j == nch - 1) umma_commit(&ra_empty[t]);
-              }
-              umma_commit(&s1_empty[s]);
-              if (++s == STAGES) { s = 0; ph ^= 1; }
-            }
-          } else {
           for (int kb = 0; kb < kb1; ++kb) {
             mbar_wait(&s1_full[s], ph);
             tc_fence_after();
             const uint32_t sa = smem_u32(s_1 + s * S1_BYTES);
-            const uint64_t da = (BKC == 64) ? umma_desc_k128(sa) : umma_desc_k64(sa);
-            const uint64_t db = (BKC == 64) ? umma_desc_k128(sa + A1_BYTES) : umma_desc_k64(sa + A1_BYTES);
+            const uint64_t da = umma_desc_k128(sa);
+            const uint64_t db = umma_desc_k128(sa + A1_BYTES);
 #pragma unroll
             for (int k = 0; k < BKC / 16; ++k) umma_f16(d1, da + 2 * k, db + 2 * k, idesc1, (kb | k) != 0 ? 1u : 0u);
             umma_commit(&s1_empty[s]);
             if (++s == STAGES) { s = 0; ph ^= 1; }
-          }
           }
           umma_commit(&t1_full[b]);
           if (j >= 1) gemm2(j - 1);
@@ -228,7 +186,6 @@ fmb_fused_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constan
         gemm2(nch - 1);
         umma_commit(t2_full);
         t2ph ^= 1;
-        raph ^= 1;
       }
     }
   } else if (warp >= 12) {
@@ -330,21 +287,18 @@ bool fmb_fused_ok(int Cin, int Cmid, int Cout, int ksize, int stride, int pad, i
   if (en < 0) { const char* e = getenv("SB_FMB_FUSED"); en = e ? (e[0] - '0') : 1; }
   if (!en) return false;
   if (ksize != 3 || pad != 1 || (stride != 1 && stride != 2) || act1 != ACT_HARDSWISH || act2 != ACT_NONE) return false;
-  // Cin = 32 (stage 0, block 0) is instantiated and correct (bit-identical) but not faster than the two separate kernels: 1.38 vs
-  // 1.33 ms at B = 32 with per-chunk 64-byte tap boxes, and still no gain with resident tap tiles + tap-pair weight boxes (whole
-  // forward 18.52 vs 18.31 ms) -> opt-in with SB_FMB_FUSED=2
-  if (Cin == 32 && en < 2) return false;
-  if (Cin != 32 && Cin != 64 && Cin != 128) return false;
+  // Cin = 32 (stage 0, block 0) stays on the two separate kernels: fused, it measured slower (1.38 vs 1.33 ms at B = 32)
+  if (Cin != 64 && Cin != 128) return false;
   if (Cmid % 128 || Cmid < 128 || Cmid > 1024) return false;
   return Cout == 64 || Cout == 128;
 }
 
-template <typename T, int BKC, int COUT, int STAGES, int NW2>
+template <typename T, int COUT, int STAGES, int NW2>
 static int launch_fmb(int dtype, const void* in, const void* w1, const void* w2, const FmbParams& fp, cudaStream_t st) {
-  constexpr bool RES_A = (BKC == 32);
-  constexpr size_t S1 = RES_A ? static_cast<size_t>(128 * 64 * 2) : static_cast<size_t>(128 * BKC * 2) * 2;
-  const size_t SMEM = (RES_A ? 9 * 128 * 32 * 2 : 0) + STAGES * S1 + 2 * 32768 + NW2 * (COUT * 256) + (fp.Cmid + COUT) * 4 + 512 + 1024;
-  auto kern = fmb_fused_kernel<T, BKC, COUT, STAGES, NW2>;
+  constexpr int BKC = 64;
+  constexpr size_t S1 = static_cast<size_t>(128 * BKC * 2) * 2;
+  const size_t SMEM = STAGES * S1 + 2 * 32768 + NW2 * (COUT * 256) + (fp.Cmid + COUT) * 4 + 512 + 1024;
+  auto kern = fmb_fused_kernel<T, COUT, STAGES, NW2>;
   if (cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM) != cudaSuccess) {
     cudaGetLastError();
     set_error("fmb_fused: cudaFuncSetAttribute(smem=%zu) failed", SMEM);
@@ -353,8 +307,7 @@ static int launch_fmb(int dtype, const void* in, const void* w1, const void* w2,
   CUtensorMap ma, m1, m2;
   int rc = make_tma_nhwc(&ma, dtype, in, fp.n_img, fp.H, fp.W, fp.Cin, BKC, 16, 8, fp.stride, BKC * 2);
   if (rc) return rc;
-  rc = RES_A ? make_tma_2d(&m1, dtype, w1, fp.Cmid, 9 * fp.Cin, 9 * fp.Cin, 128)      // [128 x 64] boxes over tap pairs, 128B swizzle
-             : make_tma_2d_sw(&m1, dtype, w1, fp.Cmid, 9 * fp.Cin, 9 * fp.Cin, BKC, 128, BKC * 2);
+  rc = make_tma_2d_sw(&m1, dtype, w1, fp.Cmid, 9 * fp.Cin, 9 * fp.Cin, BKC, 128, BKC * 2);
   if (rc) return rc;
   rc = make_tma_2d(&m2, dtype, w2, COUT, fp.Cmid, fp.Cmid, COUT);
   if (rc) return rc;
@@ -377,10 +330,8 @@ int fmb_fused(int dtype, const void* in, const void* w1, const float* bias1, con
   fp.bias1 = bias1; fp.bias2 = bias2; fp.residual = residual; fp.out = out;
 #define FMB(T_) \
   do { \
-    if (Cin == 32 && Cout == 64) return launch_fmb<T_, 32, 64, 3, 2>(dtype, in, w1, w2, fp, st); \
-    if (Cin == 32 && Cout == 128) return launch_fmb<T_, 32, 128, 3, 1>(dtype, in, w1, w2, fp, st); \
-    if (Cout == 64) return launch_fmb<T_, 64, 64, 3, 2>(dtype, in, w1, w2, fp, st); \
-    return launch_fmb<T_, 64, 128, 3, 1>(dtype, in, w1, w2, fp, st); \
+    if (Cout == 64) return launch_fmb<T_, 64, 3, 2>(dtype, in, w1, w2, fp, st); \
+    return launch_fmb<T_, 128, 3, 1>(dtype, in, w1, w2, fp, st); \
   } while (0)
   if (dtype == DT_BF16) FMB(__nv_bfloat16); else FMB(__half);
 #undef FMB

@@ -50,10 +50,6 @@ struct GemmArgs {
 // M <= 16 rows: mma.sync kernel without the tcgen05 set-up costs (gemm_skinny.cu); gemm_launch routes to it when it applies.
 bool gemm_skinny_ok(const GemmArgs& a);
 int gemm_skinny_launch(const GemmArgs& a, cudaStream_t stream);
-// Several dependent skinny GEMMs in one persistent launch with grid-wide barriers between them (gemm_chain.cu); `bar` = 3
-// zero-initialised uint32 owned by the caller (re-armed by the kernel).  phases[i].force_bn > 0 fixes that phase's tile width.
-int gemm_chain_launch(const GemmArgs* phases, int n, unsigned int* bar, cudaStream_t stream);
-int gemm_chain_bn(int M, int N, int swiglu);
 // Tile width gemm_launch will use for an argmax-epilogue launch of this shape (partials per row = ceil(N / width)).
 int gemm_argmax_tile(int M, int N);
 

@@ -393,11 +393,6 @@ __device__ __forceinline__ void epilogue_stage_bias(const GemmKParams& p, float*
     sbias[j] = (p.bias && n_col0 + j < p.N) ? __ldg(p.bias + n_col0 + j) : 0.f;
 }
 
-__device__ __forceinline__ void epilogue_stage_bias_rt(const GemmKParams& p, float* sbias, int epi_tid, int n_col0, int bn) {
-  for (int j = epi_tid; j < bn; j += EPI_WARPS * 32)
-    sbias[j] = (p.bias && n_col0 + j < p.N) ? __ldg(p.bias + n_col0 + j) : 0.f;
-}
-
 // Runtime -> compile-time dispatch on (act, swiglu); once per tile, outside every loop.  ng = 32-column groups in the tile.
 template <typename T, typename RowFn>
 __device__ __forceinline__ void epilogue_tile_rt(uint32_t taddr, const GemmKParams& p, uint8_t* stage, const float* sbias,

@@ -37,8 +37,8 @@ __device__ __forceinline__ void tile_coords(int tile, int m_blocks, int n_blocks
   nb = r / gsz;
 }
 
-template <typename T, int BN, int STAGES, int MINB = 1>
-__global__ void __launch_bounds__(384, MINB)
+template <typename T, int BN, int STAGES>
+__global__ void __launch_bounds__(384, 1)
 gemm_tn_kernel(const __grid_constant__ CUtensorMap tma_a, const __grid_constant__ CUtensorMap tma_b,
                const GemmKParams p) {
   constexpr int BM = 128, BK = 64;
@@ -405,13 +405,12 @@ int make_tma_nhwc(CUtensorMap* map, int dtype, const void* base, int N, int H, i
   return 0;
 }
 
-template <typename T, int BN, int STAGES, int MINB = 1>
+template <typename T, int BN, int STAGES>
 static int launch_cfg(const GemmArgs& a, cudaStream_t stream) {
   constexpr uint32_t STAGE_BYTES = 128 * 64 * 2 + BN * 64 * 2;
   constexpr size_t SMEM = STAGES * STAGE_BYTES + 1024 /*align slack*/ + 256 /*barriers*/ + epi_smem_bytes<BN>();
-  static_assert(MINB == 1 || (MINB * (SMEM + 1024) <= 228 * 1024 && MINB * 2 * BN <= 512), "co-resident CTAs must fit smem and TMEM");
   static bool attr_set = false;
-  auto kern = gemm_tn_kernel<T, BN, STAGES, MINB>;
+  auto kern = gemm_tn_kernel<T, BN, STAGES>;
   if (!attr_set) {
     cudaError_t e = cudaFuncSetAttribute(kern, cudaFuncAttributeMaxDynamicSharedMemorySize, (int)SMEM);
     if (e != cudaSuccess) {
@@ -442,34 +441,15 @@ static int launch_cfg(const GemmArgs& a, cudaStream_t stream) {
   p.am_val = a.am_val; p.am_idx = a.am_idx; p.am_sum = a.am_sum; p.am_ld = a.am_ld; p.store_c = a.store_c;
   int m_blocks = (a.M + 127) / 128, n_blocks = (a.N + BN - 1) / BN;
   int tiles = m_blocks * n_blocks;
-  int grid = tiles < MINB * num_sms() ? tiles : MINB * num_sms();
+  int grid = tiles < num_sms() ? tiles : num_sms();
   if (launch_pdl(kern, dim3(grid), dim3(384), SMEM, stream, ma, mb, p) != cudaSuccess) { /* reported by launch_ok */ }
   return launch_ok();
-}
-
-// Short-K GEMMs with an activation (detection's 1x1 expand convs, K = 128 ... 256; the Swin fc1 of the narrow stages) are bound
-// by their epilogue, and the epilogue by latency: 8 epilogue warps (2 per sub-partition) run at ~0.13 IPC each
-// (profiles/r02_gemm_expand_epilogue_ncu.md).  For these, 128 x 128 tiles with a 2-stage ring need 100 KB of shared memory and
-// 256 TMEM columns, so TWO CTAs fit on an SM (80 registers per thread: ~150 bytes of spills in the epilogue) and 16 epilogue
-// warps hide each other's tcgen05.ld / staging latencies.  The per-element arithmetic and the k order do not change (bit-identical,
-// tests/test_ops_gpu.py::test_gemm_two_ctas_per_sm_config).  MEASURED: the detection forward gets slower with it (19.10 vs 18.37 ms
-// at B = 32): N = 128 MMAs cost the same ~115 cycles as N = 256 ones and the 2-stage ring exposes TMA latency, which outweighs the
-// extra epilogue warps — so the epilogue is not simply starved of warps.  Kept behind SB_GEMM_2CTA=1.
-static bool two_cta_ok(const GemmArgs& a) {
-  static int en = -1;
-  if (en < 0) { const char* e = getenv("SB_GEMM_2CTA"); en = (e && e[0] == '1') ? 1 : 0; }   // opt-in: measured slower, see above
-  if (!en || a.force_bn != 0) return false;
-  if (a.K > 256 || a.act == ACT_NONE || a.swiglu || a.group_k || a.out_f32 || a.rowscale || a.ssq_inline || a.am_val) return false;
-  if (a.N % 128 || a.N < 256) return false;
-  const long long tiles = static_cast<long long>((a.M + 127) / 128) * (a.N / 128);
-  return tiles >= 4LL * num_sms();
 }
 
 template <typename T>
 static int launch_typed(const GemmArgs& a, cudaStream_t stream) {
   int bn = a.force_bn;
   if (bn >= 1000) return gemm_splitk_launch(a, bn / 1000, bn % 1000, stream);   // forced split-K: 1000 * pk + BN
-  if (two_cta_ok(a)) return launch_cfg<T, 128, 2, 2>(a, stream);
   if (bn == 0 && a.allow_splitk && splitk_enabled() && !a.rowscale && !a.ssq_inline && !a.am_val) {
     int sbn = 0;
     const int pk = splitk_plan(a, &sbn);

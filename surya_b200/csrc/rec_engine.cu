@@ -8,7 +8,6 @@
 #include "ops.cuh"
 #include "sb_ptx.cuh"
 
-#include <cstdlib>
 #include <cstring>
 #include <string>
 #include <vector>
@@ -40,12 +39,6 @@ struct sb_rec_engine {
   // lm_head argmax partials [rows, am_ld]: (max, argmax, sum exp) per 128 x am_bn logit tile
   float* am_val = nullptr; int* am_idx = nullptr; float* am_sum = nullptr;
   int am_ld = 0, am_bn = 0;
-  // gemm_chain (o_proj -> gate/up -> down -> next qkv in one persistent launch): barrier counters + switch.  OFF by default:
-  // measured 50.7 us per layer chain vs 46.4 us for the four PDL-chained launches (profiles/r02_chain_timeline.md) — each phase
-  // still pays ~1.5 us first-tile latency + ~2 us grid barrier, and the down projection loses its split-K kernel.  $SB_CHAIN=1
-  // or sb_rec_set_option("chain", 1) turns it on.
-  unsigned int* chain_bar = nullptr;
-  int use_chain = 0;
   int qkv_w_enc = 0, qkv_w_dec = 0;
   // CUDA graph cache for decode_steps
   cudaGraphExec_t graph_exec = nullptr;
@@ -236,19 +229,6 @@ static int run_decoder_prefill(sb_rec_engine* e, const long long* ids, int n_tok
   return run_heads(e, e->xl, n_seq, out, st);
 }
 
-static GemmArgs chain_phase(const sb_rec_engine* e, const void* A, int lda, const void* Wt, int ldw, void* C, int ldc, int M, int N,
-                            int K, const void* bias_f32, const void* residual, int ldr, int act, int swiglu, int norm) {
-  GemmArgs a;
-  a.dtype = e->c.dtype;
-  a.A = A; a.lda = lda; a.W = Wt; a.ldw = ldw; a.C = C; a.ldc = ldc;
-  a.M = M; a.N = N; a.K = K;
-  a.bias = static_cast<const float*>(bias_f32);
-  a.residual = residual; a.ldr = ldr; a.act = act; a.swiglu = swiglu;
-  a.w_constant = 1;
-  if (norm) { a.ssq_inline = 1; a.ssq_eps = e->c.rms_eps; a.ssq_k = K; }
-  return a;
-}
-
 // One greedy decode step for `B` rows: 5 launches per layer (qkv GEMM -> attention -> o GEMM -> gate/up GEMM -> down GEMM)
 // + lm_head + tail.  ids == nullptr means e->x already holds the input embeddings (written by the previous step's tail).
 static int run_decode_step(sb_rec_engine* e, const long long* ids, const int* slot, const int* pos, int B, const HeadOut& out,
@@ -259,31 +239,6 @@ static int run_decode_step(sb_rec_engine* e, const long long* ids, const int* sl
   const int dt = c.dtype;
   void* x = e->x;
   if (ids) CK(embed_rows(dt, ids, e->W(SB_RW_EMBED), x, D, B, D, st));
-  if (e->use_chain && B <= 256) {
-    // 2 launches per layer: decode attention, then ONE persistent kernel for o_proj -> gate/up -> down -> the next layer's qkv
-    // (grid barriers between the four GEMMs, gemm_chain.cu); the first qkv and the heads are separate launches
-    CK(linear(e, x, D, e->WD(0, SB_RWD_QKV_W), D, e->qkv, Q, B, Q, D, e->WD(0, SB_RWD_QKV_B), nullptr, 0, ACT_NONE, 0, st, 0, 2));
-    for (int l = 0; l < c.dec_layers; ++l) {
-      DecodeAttnArgs a;
-      a.dtype = dt; a.qkv = e->qkv; a.ld = Q; a.kcache = e->kc(l); a.vcache = e->vc(l); a.slot = slot; a.pos = pos;
-      a.inv_freq = static_cast<const float*>(e->W(SB_RW_DEC_INV_FREQ));
-      a.out = e->ao; a.ldo = nh * hd; a.batch = B; a.n_heads = nh; a.n_kv_heads = nkv; a.head_dim = hd; a.s_max = c.s_max;
-      a.scale = 1.0f / sqrtf(static_cast<float>(hd));
-      CK(decode_attn(a, st));
-      GemmArgs ph[4];
-      int n = 0;
-      ph[n++] = chain_phase(e, e->ao, nh * hd, e->WD(l, SB_RWD_O_W), nh * hd, x, D, B, D, nh * hd, nullptr, x, D, ACT_NONE, 0, 0);
-      ph[n++] = chain_phase(e, x, D, e->WD(l, SB_RWD_GU_W), D, e->act, c.dec_inter_pad, B, 2 * c.dec_inter_pad, D, nullptr, nullptr, 0,
-                            ACT_SILU, 1, 1);
-      ph[n++] = chain_phase(e, e->act, c.dec_inter_pad, e->WD(l, SB_RWD_DOWN_W), c.dec_inter_pad, x, D, B, D, c.dec_inter_pad, nullptr,
-                            x, D, ACT_NONE, 0, 0);
-      if (l + 1 < c.dec_layers)
-        ph[n++] = chain_phase(e, x, D, e->WD(l + 1, SB_RWD_QKV_W), D, e->qkv, Q, B, Q, D, e->WD(l + 1, SB_RWD_QKV_B), nullptr, 0,
-                              ACT_NONE, 0, 1);
-      CK(gemm_chain_launch(ph, n, e->chain_bar, st));
-    }
-    return run_heads(e, x, B, out, st);
-  }
   for (int l = 0; l < c.dec_layers; ++l) {
     CK(linear(e, x, D, e->WD(l, SB_RWD_QKV_W), D, e->qkv, Q, B, Q, D, e->WD(l, SB_RWD_QKV_B), nullptr, 0, ACT_NONE, 0, st, 0,
               /*norm=*/2));
@@ -319,7 +274,6 @@ int sb_rec_create(const sb_rec_config* cfg, const void* const* weights, int n_we
   auto* e = new sb_rec_engine();
   e->c = *cfg;
   e->w.assign(weights, weights + n_weights);
-  if (const char* ev = getenv("SB_CHAIN")) e->use_chain = (ev[0] != '0');
   const sb_rec_config& c = e->c;
   const size_t es = e->esz;
   const size_t R = static_cast<size_t>(c.max_patches > c.max_tokens ? c.max_patches : c.max_tokens);
@@ -339,7 +293,7 @@ int sb_rec_create(const sb_rec_config* cfg, const void* const* weights, int n_we
       (size_t)c.max_patches * c.patch_dim_pad * es, nm * c.merge_unit * c.enc_hidden * es,  // x0 m1
       nm * c.enc_out_hidden * es, rows_out * c.dec_hidden * es, rows_out * c.vocab * es,   // feat xl logits
       kv_bytes, kv_bytes,
-      rows_out * 8, rows_out * 4, rows_out * 6 * 8, rows_out, rows_out * 8, 256, 256, 256,
+      rows_out * 8, rows_out * 4, rows_out * 6 * 8, rows_out, rows_out * 8, 256, 256,
       R * 4, am_elems * 4, am_elems * 4, am_elems * 4};
   size_t total = 0;
   for (size_t s : sizes) total += al256(s);
@@ -353,7 +307,7 @@ int sb_rec_create(const sb_rec_config* cfg, const void* const* weights, int n_we
   uint8_t* p = e->arena;
   void** slots[] = {&e->x, &e->nbuf, &e->qkv, &e->ao, &e->act, &e->x0, &e->m1, &e->feat, &e->xl, &e->logits,
                     &e->kcache, &e->vcache, (void**)&e->st_tok, (void**)&e->st_score, (void**)&e->st_bbox,
-                    (void**)&e->st_done, (void**)&e->st_next, (void**)&e->st_step, (void**)&e->st_counter, (void**)&e->chain_bar,
+                    (void**)&e->st_done, (void**)&e->st_next, (void**)&e->st_step, (void**)&e->st_counter,
                     (void**)&e->rs, (void**)&e->am_val, (void**)&e->am_idx, (void**)&e->am_sum};
   for (size_t i = 0; i < sizeof(sizes) / sizeof(sizes[0]); ++i) {
     *slots[i] = p;
@@ -500,18 +454,6 @@ int sb_rec_set_sched(sb_rec_engine* e, int* gen_count, long long* ring, unsigned
   return 0;
 }
 
-int sb_rec_set_option(sb_rec_engine* e, const char* name, int value) {
-  if (!e || !name) { set_error("sb_rec_set_option: null argument"); return -1; }
-  std::string n(name);
-  if (n == "chain") {
-    if ((value != 0) != (e->use_chain != 0) && e->graph_exec) { cudaGraphExecDestroy(e->graph_exec); e->graph_exec = nullptr; }
-    e->use_chain = value != 0;
-    return 0;
-  }
-  set_error("sb_rec_set_option: unknown option '%s'", name);
-  return -2;
-}
-
 int sb_rec_debug_copy(sb_rec_engine* e, const char* name, void* dst, size_t bytes, void* stream) {
   if (!e || !name || !dst) { set_error("sb_rec_debug_copy: null argument"); return -1; }
   std::string n(name);
@@ -523,7 +465,6 @@ int sb_rec_debug_copy(sb_rec_engine* e, const char* name, void* dst, size_t byte
   else if (n == "qkv") src = e->qkv;
   else if (n == "kcache") src = e->kcache;
   else if (n == "vcache") src = e->vcache;
-  else if (n == "chain_bar") src = e->chain_bar;
   if (!src) { set_error("sb_rec_debug_copy: unknown workspace '%s'", name); return -2; }
   cudaError_t ce = cudaMemcpyAsync(dst, src, bytes, cudaMemcpyDeviceToDevice, static_cast<cudaStream_t>(stream));
   if (ce != cudaSuccess) { set_error("sb_rec_debug_copy: %s", cudaGetErrorString(ce)); return -3; }

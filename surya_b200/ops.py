@@ -72,41 +72,6 @@ def gemm(a, w, bias=None, residual=None, act="none", swiglu=False, out=None, out
     return out
 
 
-class _GemmPhaseC(ctypes.Structure):
-    _fields_ = [("A", c_void_p), ("lda", c_int), ("W", c_void_p), ("ldw", c_int), ("C", c_void_p), ("ldc", c_int),
-                ("M", c_int), ("N", c_int), ("K", c_int), ("bias", c_void_p), ("residual", c_void_p), ("ldr", c_int),
-                ("act", c_int), ("swiglu", c_int), ("rms_eps", c_float), ("force_bn", c_int)]
-
-
-def gemm_chain(phases, barrier, timeline=None):
-    """sb_gemm_chain: up to 4 dependent skinny GEMMs in one persistent launch.  phases: dicts with a, w, out and optionally
-    bias, residual, act, swiglu, rms_eps, force_bn (same meaning as gemm()); barrier: zeroed int32[4] device tensor."""
-    lib = _lib.load()
-    arr = (_GemmPhaseC * len(phases))()
-    keep = []
-    for q, ph in zip(arr, phases):
-        a, w, out = ph["a"], ph["w"], ph["out"]
-        res = ph.get("residual")
-        q.A, q.lda, q.W, q.ldw, q.C, q.ldc = a.data_ptr(), _rowmajor(a), w.data_ptr(), _rowmajor(w), out.data_ptr(), _rowmajor(out)
-        q.M, q.N, q.K = a.shape[0], w.shape[0], a.shape[1]
-        q.bias = ph["bias"].data_ptr() if ph.get("bias") is not None else None
-        q.residual = res.data_ptr() if res is not None else None
-        q.ldr = _rowmajor(res) if res is not None else 0
-        q.act, q.swiglu = ACT[ph.get("act", "none")], 1 if ph.get("swiglu") else 0
-        q.rms_eps = float(ph.get("rms_eps") or 0.0)
-        q.force_bn = int(ph.get("force_bn", 0))
-        keep.append((a, w, out, res))
-    if timeline is not None:
-        check(lib.sb_gemm_chain_timeline(dt_code(phases[0]["a"].dtype), arr, c_int(len(phases)), ptr(barrier), ptr(timeline),
-                                         stream_ptr()), "sb_gemm_chain_timeline")
-        return
-    check(lib.sb_gemm_chain(dt_code(phases[0]["a"].dtype), arr, c_int(len(phases)), ptr(barrier), stream_ptr()), "sb_gemm_chain")
-
-
-def gemm_chain_bn(M, N, swiglu=False):
-    return int(_lib.load().sb_gemm_chain_bn(c_int(M), c_int(N), c_int(1 if swiglu else 0)))
-
-
 def row_rstd(x, eps=1e-6, src_rows=None):
     """fp32 [rows]: rsqrt(mean(x^2) + eps) per row, summed in the order the GEMM's in-kernel pass uses."""
     lib = _lib.load()

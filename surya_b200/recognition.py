@@ -379,11 +379,6 @@ class RecEngine:
                                      ptr(out["done"]), ptr(out["next_ids"]), stream_ptr()), "sb_rec_decode")
         return out
 
-    def set_option(self, name: str, value: int):
-        """Engine switches (sb_rec_set_option): "chain" = run each decoder layer's four dependent GEMMs of a decode step as one
-        persistent gemm_chain launch."""
-        check(self.lib.sb_rec_set_option(self._h, name.encode(), c_int(int(value))), "sb_rec_set_option")
-
     def decode_steps(self, ids_io: torch.Tensor, slot: torch.Tensor, pos_io: torch.Tensor, n_steps: int,
                      hist: Optional[dict] = None, use_graph: bool = True, max_pos: Optional[int] = None):
         """n_steps greedy steps on the device; ids_io / pos_io advance in place. Returns step-major histories.

@@ -379,7 +379,7 @@ def test_fused_kernels_equal_unfused_ops(built_lib, switch, size, tmp_path):
     import sys
 
     outs = {}
-    on = "2" if switch == "SB_FMB_FUSED" else "1"      # 2 = also the Cin = 32 instance, which is off by default (not faster)
+    on = "1"
     for val in (on, "0"):
         path = tmp_path / f"variant{val}.pt"
         code = (f"import sys, torch; sys.path.insert(0, {str(ROOT)!r}); sys.path.insert(0, {str(ROOT / 'tests')!r});"

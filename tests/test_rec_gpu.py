@@ -393,36 +393,6 @@ def test_predictor_trace_replay_gpu(built_lib):
     eng.close()
 
 
-def test_gemm_chain_decode_path_matches_separate_launches(built_lib):
-    """The optional persistent-chain decode path (sb_rec_set_option("chain", 1)) against the default path: same tokens and
-    boxes for every crop through the device-side loop (the down projection sums in a different fp32 order — split-K kernel vs
-    plain tiles — so equality is required on the discrete outputs and a tight bound on the scores); no barrier timeout."""
-    from surya_b200.config import tiny_rec
-    from surya_b200.recognition import RecognitionRunner
-    from surya_b200.synth import rec_state_dict, rec_synthetic_crops
-
-    cfg = tiny_rec()
-    eng = _engine(cfg, rec_state_dict(cfg, seed=0), torch.float16, max_slots=16, s_max=160, max_patches=4096, max_tokens=1024)
-    crops = [rec_synthetic_crops(1, 48, 300 + 70 * i, seed=40 + i)[0] for i in range(6)]
-    runner = RecognitionRunner(eng, batch_size=6, max_tokens=12)
-    t0, s0, b0 = runner.run(crops, fixed_steps=True)
-    eng.set_option("chain", 1)
-    t1, s1, b1 = runner.run(crops, fixed_steps=True)
-    eng.set_option("chain", 0)
-    bar = torch.zeros(4, dtype=torch.int32, device="cuda")
-    from surya_b200._lib import check, ptr, stream_ptr
-    import ctypes
-    check(eng.lib.sb_rec_debug_copy(eng._h, b"chain_bar", ptr(bar), ctypes.c_size_t(12), stream_ptr()), "debug_copy")
-    torch.cuda.synchronize()
-    assert bar.tolist()[:3] == [0, 0, 0], f"chain barrier state {bar.tolist()}"
-    same = sum(a == b for a, b in zip(t0, t1))
-    assert same >= 5, f"only {same}/6 crops decode identically with the chain path"
-    for a, b, sa, sb_ in zip(t0, t1, s0, s1):
-        if a == b:
-            assert np.allclose(sa, sb_, atol=2e-3)
-    eng.close()
-
-
 def test_capacity_and_bounds_are_loud(built_lib):
     """ADVICE r1: decode past s_max must raise (never write into a neighbour's KV rows), the runner must chunk prefills by
     engine capacity and give slots back when a prefill fails."""
